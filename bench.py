@@ -4,6 +4,7 @@
     python bench.py --impl reference --steps 3 --warmup 1          # the CPU ref path (oracle port) on the host cores
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port P bench.py --gpus 8 ...
     python bench.py --workload chain                               # only the modulated-conv synthesis chain (round-1 early workload)
+    python bench.py --steps 10 --warmup 3 --dump-outputs DIR       # also write what the last timed step returned, as DIR/<name>.npy
 
 One "step" = one batch (default 32 images per GPU) through `GeneratorFull_v20.forward` (pgpp_b200.training.generator, same
 state-dict as the reference): const / style encoders, mapping, synthesis blocks b8..b512, SPADE blocks and the texture branch --
@@ -25,6 +26,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -33,6 +35,26 @@ if ROOT not in sys.path:
 
 W_DIM = 512
 RES = 512
+DUMP_BYTES = 64 * 2 ** 20
+
+
+def dump_outputs(out_dir, outputs):
+    """Write `outputs` (name -> tensor, what the timed step returned) as out_dir/<name>.npy, float64 as float64 and every other dtype
+    as float32.  Above DUMP_BYTES in all, every output keeps the same rows of its leading (batch) dimension, drawn with a fixed seed, so
+    that two builds run with the same arguments can be compared output for output."""
+    arrays = {name.replace('/', '_'): t.detach().to(torch.float64 if t.dtype == torch.float64 else torch.float32) for name, t in outputs.items()}
+    total = sum(a.numel() * a.element_size() for a in arrays.values())
+    if total > DUMP_BYTES:
+        batch = {a.shape[0] for a in arrays.values()}
+        assert len(batch) == 1, f'outputs of {total} bytes without a common batch dimension to sample: {sorted(batch)}'
+        batch = batch.pop()
+        keep = DUMP_BYTES * batch // total
+        assert keep >= 1, f'one batch row of the outputs is larger than {DUMP_BYTES} bytes'
+        rows = torch.randperm(batch, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        arrays = {name: a.index_select(0, rows.to(a.device)) for name, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f'{name}.npy'), a.cpu().numpy())
 
 
 def build_chain(device, resolution=RES):
@@ -375,9 +397,10 @@ def train_inputs_to_device(u8, device):
                 gt_parsing=u8['gt_parsing'].to(device, non_blocking=True).float())
 
 
-def train_leg(steps, warmup, batch, precision, device, rank, world, fp16_res=3):
+def train_leg(steps, warmup, batch, precision, device, rank, world, fp16_res=3, dump_dir=None):
     """BASELINE configs[4]: the G + D + D_parsing training iteration with R1, data-parallel (DDP gradient all-reduce over NCCL when
-    world > 1).  Returns the per-rank measurement dict (times already max-reduced over ranks)."""
+    world > 1).  Returns the per-rank measurement dict (times already max-reduced over ranks).  With `dump_dir`, rank 0 writes the
+    statistics the last timed iteration returned there (dump_outputs)."""
     import torch.distributed as dist
     ts = importlib.import_module('pgpp_b200.training.training_step')
     cg = importlib.import_module('pgpp_b200.torch_utils.ops.conv2d_gradfix')
@@ -411,8 +434,11 @@ def train_leg(steps, warmup, batch, precision, device, rank, world, fp16_res=3):
         step(data)
     torch.cuda.reset_peak_memory_stats(device)
     l0 = custom_ops.launch_count()
-    ms = timed(lambda: step(data), steps)
+    last = {}
+    ms = timed(lambda: last.update(step(data)), steps)
     launches = (custom_ops.launch_count() - l0) // steps
+    if dump_dir is not None and rank == 0:
+        dump_outputs(dump_dir, last)
     # per-phase split on rank 0 (CUDA events around each phase of one more iteration)
     phase_ms = {}
     for ph in dict.fromkeys(p['name'] for p in step.phases):
@@ -461,7 +487,7 @@ def run_train(args):
     torch.backends.cuda.matmul.allow_tf32 = False
     batch = args.batch if args.batch != 32 else 8
     with ClockSampler(local) as clocks:
-        r = train_leg(args.steps, args.warmup, batch, args.precision, device, rank, world, fp16_res=args.fp16_res)
+        r = train_leg(args.steps, args.warmup, batch, args.precision, device, rank, world, fp16_res=args.fp16_res, dump_dir=args.dump_outputs)
     if rank == 0:
         line = {'metric': 'training_512px_images_per_sec', 'value': r['images_per_sec'], 'unit': 'images/s', 'n_gpus': world,
                 'steps': args.steps, 'warmup': max(args.warmup, 3), 'ms_per_step': r['ms_per_step'], 'higher_is_better': True,
@@ -564,6 +590,9 @@ def run_ours(args):
     launches = custom_ops.launch_count() - launches0
     if graphed is not None:
         launches = launches_per_step * args.steps
+    if args.dump_outputs and rank == 0:
+        names = ('img', 'finetune_img', 'pred_parsing') if gen_mode else ('img', 'pred_parsing', 'tex')
+        dump_outputs(args.dump_outputs, dict(zip(names, out)))
 
     # ---- end to end through the pipeline API (pinned host in, image back to host) ----
     if gen_mode:
@@ -816,7 +845,14 @@ def main():
     ap.add_argument('--skip-cpu', action='store_true', help='skip the CPU baseline / parity leg')
     ap.add_argument('--no-graph', action='store_true', help='generator workload: time eager launches instead of CUDA-graph replay (GraphedGenerator)')
     ap.add_argument('--no-ops', action='store_true', help='generator workload: skip the op microbench sweep (the `ops` key, BASELINE configs[3])')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step returned as DIR/<name>.npy (float32 / float64; at most 64 MB in all, a fixed '
+                         'seeded choice of batch rows when the outputs are larger)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of this package\'s kernels (--impl ours)')
     if args.impl == 'reference':
         run_reference(args)
     elif args.workload == 'train':
