@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-typedef enum { PGPP_F32 = 0, PGPP_F16 = 1, PGPP_BF16 = 2, PGPP_F64 = 3 } pgpp_dtype;
+typedef enum { PGPP_F32 = 0, PGPP_F16 = 1, PGPP_BF16 = 2, PGPP_F64 = 3, PGPP_E4M3 = 4 } pgpp_dtype;   /* E4M3: fp8 operand format only */
 
 typedef enum {
     PGPP_OK = 0,
@@ -106,6 +106,11 @@ PGPP_API int pgpp_pack_activations_slice(const void* x, const int64_t size[4], c
 PGPP_API int pgpp_pack_activations_f16(const void* x, const int64_t size[4], const int64_t stride[4], int dtype,
                           const float* scale, void* out, int c_pad, int c_total, int c_off, void* stream);
 
+/* Same with ONE part of e4m3 bytes (the fp8 inference precision, operand_e4m3 of the conv descriptor): unit scale, round to nearest
+ * even, satfinite (|v| > 448 saturates to +-448).  c_total, c_off and c_pad are counted in channels = bytes. */
+PGPP_API int pgpp_pack_activations_e4m3(const void* x, const int64_t size[4], const int64_t stride[4], int dtype,
+                          const float* scale, void* out, int c_pad, int c_total, int c_off, void* stream);
+
 /* Gradient of a bias_act that was fused into a convolution's epilogue, written straight into the operand format of the data- /
  * weight-gradient kernels: out = pgpp_pack_activations(dy * act'(.) * gain, zero where the clamp was active), act'(.) and the clamp
  * gate taken from the saved OUTPUT y - what BiasActCudaGrad.forward (bias_act.py:170-186, bias_act.cu:38-146 with grad = 1)
@@ -123,6 +128,14 @@ PGPP_API int pgpp_pack_act_gradient_tiles(int h, int w);
 PGPP_API int pgpp_modulate_weights(const float* master, const float* s, void* out, int n, int64_t rows, int c_pad, int c_in,
                           int parts, void* stream);
 
+/* e4m3 weight operand of the fp8 inference precision, shared (s == NULL, n == 1) or per sample (the style modulation w * s[n]):
+ *   v[n][t][g][c]   = master[t][g][c] * s[n][c]   (c < c_in; zero beyond),   master float32 [taps][o_rows][c_pad]
+ *   scale[n][g]     = max_{t, c} |v[n][t][g][c]| / 448                        (one scale per GEMM column; 0 for an all-zero column)
+ *   out[n][t][g][c] = e4m3(v / scale[n][g])   round to nearest even, satfinite (0 where scale == 0)
+ * out: n * taps * o_rows * c_pad bytes.  The convolution multiplies its accumulator by scale (pgpp_conv_desc.wscale). */
+PGPP_API int pgpp_quantize_weights_e4m3(const float* master, const float* s, int n, int taps, int o_rows, int c_pad, int c_in,
+                          void* out, float* scale, void* stream);
+
 /* Weight operand packing, one launch (replaces the eager packing the round-1 Python shim did with library ops; there is no
  * reference counterpart: cuDNN consumes [O, I, kh, kw] directly at conv2d_gradfix.py:112-114):
  *   out[part][tap][o_off + row][c]  = split part `part` of  scale * W'[row, c, tap]      (zero for row / c beyond the tensor)
@@ -135,7 +148,8 @@ PGPP_API int pgpp_modulate_weights(const float* master, const float* s, void* ou
  * with k the 4x4 FIR `fir` (device, float32, row-major; flipped unless flip_filter, upfirdn2d.py:193-196) and w_f the flipped /
  * unflipped kernel.  operand_f16 != 0 writes IEEE half instead of bfloat16 (parts must be 1): the fp16 layers of the
  * discriminator (networks.py:634,647) run native f16 MMAs.  The destination has o_rows rows per tap; rows outside
- * [o_off, o_off + rows) are left untouched (zero them once, or pack several tensors side by side: gamma | beta). */
+ * [o_off, o_off + rows) are left untouched (zero them once, or pack several tensors side by side: gamma | beta).  out may be NULL when
+ * master is given (the fp8 route quantizes master with pgpp_quantize_weights_e4m3). */
 PGPP_API int pgpp_pack_weights(const void* w, int w_dtype, const int64_t w_size[4], const int64_t w_stride[4], int transpose_io, int flip,
                       float scale, int phases, int phase_stride, const float* fir, int flip_filter,
                       void* out, float* master, int parts, int operand_f16, int o_rows, int o_off, int c_pad, void* stream);
@@ -207,7 +221,8 @@ typedef struct {
     float alpha, gain, clamp;
     /* output tensor, logical [N, o, out_h, out_w] with element strides (any layout) */
     void* out;
-    int32_t out_dtype;              /* PGPP_F32 / PGPP_BF16 / PGPP_F16 */
+    int32_t out_dtype;              /* PGPP_F32 / PGPP_BF16 / PGPP_F16; PGPP_E4M3 (e4m3 operands only): the channels-innermost e4m3
+                                       operand format of the next conv, from the lean operand-format epilogue */
     int32_t out_h, out_w;
     int64_t out_stride[4];
     int32_t accumulate;             /* nonzero: out += result (used for `img = img + y`, networks.py:2190) */
@@ -232,6 +247,12 @@ typedef struct {
      * tile, conv_w and conv_h multiples of the pixel tile (16 x 8, or 8 x 16 in single-slab mode), o % 16 == 0, phases == 1, no
      * accumulate; pgpp_conv2d_igemm_stats_rows reports M (0 = this launch cannot produce statistics). */
     float* stats_ws;
+    /* fp8 inference precision (operand_e4m3 != 0): act and wgt hold ONE part of e4m3 bytes (products == 1), act at unit scale, the
+     * weights of GEMM column g divided by wscale[g] (wgt_per_sample: wscale[n * o_rows + g]); the epilogue multiplies the accumulator
+     * by wscale together with dcoef.  tcgen05.mma kind::f8f6f4, channel blocks of 32 / 64 / 128 channels (one byte each). */
+    const float* wscale;
+    int32_t operand_e4m3;
+    int32_t reserved1;
 } pgpp_conv_desc;
 
 /* Implicit-GEMM convolution on the 5th-gen tensor cores (tcgen05.mma, TMEM accumulators, TMA operand

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <cuda_fp16.h>
 #include <cuda_bf16.h>
+#include <cuda_fp8.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <stdarg.h>
@@ -86,5 +87,18 @@ __device__ __forceinline__ void ffma2(f32x2& d, const f32x2 a, const f32x2 b) { 
 __device__ __forceinline__ f32x2 fadd2(const f32x2 a, const f32x2 b) { f32x2 d; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
 // bf16 pair (one 32-bit word, low half = even channel) -> packed float32 pair
 __device__ __forceinline__ f32x2 bf2_to_f32x2(uint32_t w) { return (f32x2)(w << 16) | ((f32x2)(w & 0xffff0000u) << 32); }
+
+// e4m3 operand format (the opt-in fp8 inference precision): round to nearest even, satfinite (|x| > 448 -> +-448, NaN stays NaN),
+// i.e. cvt.rn.satfinite.e4m3x2.f32.  Four values -> one 32-bit word, byte k = value k (channels ascending in memory).
+__device__ __forceinline__ uint32_t e4m3x4(float a, float b, float c, float d) {
+    const uint32_t lo = __nv_cvt_float2_to_fp8x2(make_float2(a, b), __NV_SATFINITE, __NV_E4M3);
+    const uint32_t hi = __nv_cvt_float2_to_fp8x2(make_float2(c, d), __NV_SATFINITE, __NV_E4M3);
+    return lo | (hi << 16);
+}
+// byte pair (low byte = even channel) -> two floats (exact: every e4m3 value is a half)
+__device__ __forceinline__ float2 e4m3x2_to_float2(uint32_t pair) {
+    const __half2_raw h = __nv_cvt_fp8x2_to_halfraw2((__nv_fp8x2_storage_t)(pair & 0xffffu), __NV_E4M3);
+    return __half22float2(*reinterpret_cast<const __half2*>(&h));
+}
 
 } // namespace pgpp

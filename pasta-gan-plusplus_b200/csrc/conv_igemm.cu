@@ -33,6 +33,7 @@
 #include <cuda.h>
 #include <stdlib.h>
 #include <atomic>
+#include <type_traits>
 #include "act.cuh"
 #include "tc_ptx.cuh"
 
@@ -86,7 +87,13 @@ struct IgemmParams {
                                         // arithmetic / stores, 2 without TMEM loads, 4 no MMAs issued, 8 arithmetic but no stores, 16 stores go to one
                                         // tile-sized region (no DRAM write traffic), 32 128-bit instead of 256-bit stores of the operand format, 64 no activation loads (the MMA warp
                                         // does not wait for them: MMA issue + tensor time alone)
+    const float* wscale;                // e4m3 operands: per-GEMM-column weight scale [o_rows] (per sample: [n][o_rows]), folded into the epilogue scale
 };
+
+// column scale of the e4m3 weights (fp8 inference precision) for sample n, GEMM column g
+__device__ __forceinline__ float weight_scale(const IgemmParams& p, int n, int g) {
+    return __ldg(p.wscale + (p.wgt_per_sample ? (long long)n * p.o_rows : 0ll) + g);
+}
 
 
 // ------------------------------------------------------------------------------------------------
@@ -123,7 +130,7 @@ template <> __device__ __forceinline__ float cvt_in<__half>(__half v) { return _
 
 // General epilogue of one accumulator tile for the calling warp: its 32 TMEM lanes (pixels) x columns
 // [col_begin, col_end).  Handles every option (several samples per tile, accumulate, partial chunks, any activation).
-template <int A, class OT>
+template <int A, class OT, bool F8>
 __device__ __forceinline__ void epilogue_general(const IgemmParams& p, const TileCoord tc, uint32_t tmem_tile, const PixelCoord pc,
                                                  int col_begin, int col_end) {
     const int x = tc.x0 + pc.px, y = tc.y0 + pc.py, n = tc.n0 + pc.pn;
@@ -152,6 +159,7 @@ __device__ __forceinline__ void epilogue_general(const IgemmParams& p, const Til
                 const int oc = oc0 + j;
                 float r = v[j];
                 if (p.dcoef) r *= __ldg(p.dcoef + (long long)n * p.o + oc);
+                if (F8) r *= weight_scale(p, n, g0 + j);
                 r += nz;
                 if (p.bias) r += __ldg(p.bias + oc);
                 r = act_forward<A, float>(r, alpha) * gain;
@@ -369,6 +377,8 @@ __device__ __forceinline__ void epilogue_fast(const IgemmParams& p, const TileCo
 //   v = (x - mean) * rstd * (1 + gamma) + beta,   then the consumer's pre-activation relu(v) * pre_gain,
 // and writes the bf16 expansion of v channels-innermost: the operand format of the next convolution.
 // s_cs[c] = (rstd[n, c], bias_gamma[c]), s_cs[C + c] = (mean[n, c], bias_beta[c]).
+// F8: e4m3 operands - gamma / beta are the accumulators times the weight column scales; the output is e4m3 when out_dtype says so.
+template <bool F8>
 __device__ __forceinline__ void epilogue_spade(const IgemmParams& p, const TileCoord tc, uint32_t tmem_tile, const PixelCoord pc,
                                                int half, const float2* s_cs) {
     const int C = p.o >> 1;
@@ -395,10 +405,18 @@ __device__ __forceinline__ void epilogue_spade(const IgemmParams& p, const TileC
         #pragma unroll
         for (int j = 0; j < 16; j++) {
             const float2 qg = s_cs[c0 + j], qb = s_cs[C + c0 + j];
-            const float g = __uint_as_float(rg[j]) + qg.y, b = __uint_as_float(rb[j]) + qb.y;
+            float ag = __uint_as_float(rg[j]), ab = __uint_as_float(rb[j]);
+            if (F8) { ag *= weight_scale(p, n, c0 + j); ab *= weight_scale(p, n, C + c0 + j); }
+            const float g = ag + qg.y, b = ab + qb.y;
             float r = fmaf((xv[j] - qb.x) * qg.x, 1.f + g, b);
             if (pre_gain > 0.f) r = fmaxf(r, 0.f) * pre_gain;
             v[j] = r;
+        }
+        if (F8 && p.out_dtype == PGPP_E4M3) {
+            uint8_t* const dst8 = (uint8_t*)p.out + n * p.os_n + y * p.os_h + x * p.os_w + c0;
+            *reinterpret_cast<uint4*>(dst8) = make_uint4(e4m3x4(v[0], v[1], v[2], v[3]), e4m3x4(v[4], v[5], v[6], v[7]),
+                                                         e4m3x4(v[8], v[9], v[10], v[11]), e4m3x4(v[12], v[13], v[14], v[15]));
+            continue;
         }
         for (int part = 0; part < p.out_parts; part++) {
             __align__(16) __nv_bfloat16 tmp[16];
@@ -412,7 +430,7 @@ __device__ __forceinline__ void epilogue_spade(const IgemmParams& p, const TileC
     }
 }
 
-template <class OT>
+template <class OT, bool F8>
 __device__ __forceinline__ void epilogue_dispatch(const IgemmParams& p, const TileCoord tc, uint32_t tmem_tile, const PixelCoord pc,
                                                   int col_begin, int col_end, const float2* s_cs, bool fast, float nz_pre, float* stats_row) {
     if (fast) {
@@ -431,7 +449,7 @@ __device__ __forceinline__ void epilogue_dispatch(const IgemmParams& p, const Ti
 #undef PGPP_FAST
         return;
     }
-#define PGPP_EPI(ACT) epilogue_general<ACT, OT>(p, tc, tmem_tile, pc, col_begin, col_end)
+#define PGPP_EPI(ACT) epilogue_general<ACT, OT, F8>(p, tc, tmem_tile, pc, col_begin, col_end)
     switch (p.act_fn) {
         case PGPP_ACT_LINEAR: PGPP_EPI(PGPP_ACT_LINEAR); break;
         case PGPP_ACT_RELU: PGPP_EPI(PGPP_ACT_RELU); break;
@@ -454,7 +472,8 @@ __device__ __forceinline__ void epilogue_dispatch(const IgemmParams& p, const Ti
 // STK: columns [block_n, 2 * block_n) of the accumulator hold a0 x b1 and are added to a0 x b0 + a1 x b0 (see mma_role).
 // ACC: out += result on the operand format (the residual adds y = skip + conv1(...) of ResBlock / Spade_ResBlockV4_512 without
 // leaving the format): the parts already stored are summed, the result added and the bf16 expansion written back.
-template <int A, bool STK, bool ACC>
+// F8: e4m3 operands (the column scale of the weights joins the staged scale) and e4m3 output, one part, one 128-bit store per 16 channels.
+template <int A, bool STK, bool ACC, bool F8 = false>
 __device__ __forceinline__ void epilogue_packed_role(const IgemmParams& p, uint32_t bar_base, uint32_t tmem_base, float2* s_params,
                                                      int warp, int lane) {
     const uint32_t tfull0 = bar_base + 8u * (2 * p.a_stages + 2 * p.b_stages), tempty0 = tfull0 + 16u;
@@ -465,7 +484,8 @@ __device__ __forceinline__ void epilogue_packed_role(const IgemmParams& p, uint3
     const int block_n = p.block_n, cols_per = block_n >> 1, col_begin = half * cols_per;
     const float alpha = p.alpha, gain = p.gain;
     const float cl = p.clamp >= 0.f ? p.clamp : __int_as_float(0x7f800000);      // no clamp: +-inf bounds
-    __nv_bfloat16* const out = (__nv_bfloat16*)p.out;
+    typedef typename std::conditional<F8, uint8_t, __nv_bfloat16>::type ET;
+    ET* const out = (ET*)p.out;
     const long long part_stride = p.out_part_stride;
     const int nparts = p.out_parts;
     const float* const noise = p.noise;
@@ -476,7 +496,7 @@ __device__ __forceinline__ void epilogue_packed_role(const IgemmParams& p, uint3
         return (noise && x < conv_w && y < conv_h) ? __ldg(noise + c.n0 * p.noise_stride_n + (long long)y * p.out_w + x) : 0.f;
     };
     // one 16-column chunk: scale / noise / shift / activation / clamp, bf16 expansion, 256-bit stores
-    auto chunk = [&](const uint32_t* acc, const float2* s_cs, float nz, __nv_bfloat16* dst, bool store) {
+    auto chunk = [&](const uint32_t* acc, const float2* s_cs, float nz, ET* dst, bool store) {
         float v[16];
         const float4* s_cs4 = reinterpret_cast<const float4*>(s_cs);
         #pragma unroll
@@ -495,6 +515,22 @@ __device__ __forceinline__ void epilogue_packed_role(const IgemmParams& p, uint3
             store = store && sum == 1.2345e38f;
         }
         if (!store) return;
+        if constexpr (F8) {
+            if (ACC) {
+                uint32_t prev[4];
+                asm volatile("ld.global.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(prev[0]), "=r"(prev[1]), "=r"(prev[2]), "=r"(prev[3]) : "l"(dst) : "memory");
+                #pragma unroll
+                for (int j = 0; j < 8; j++) {
+                    const float2 f = e4m3x2_to_float2(prev[j >> 1] >> (16 * (j & 1)));
+                    v[2 * j] += f.x; v[2 * j + 1] += f.y;
+                }
+            }
+            uint32_t w[4];
+            #pragma unroll
+            for (int j = 0; j < 4; j++) w[j] = e4m3x4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+            asm volatile("st.global.v4.b32 [%0], {%1, %2, %3, %4};" ::"l"(dst), "r"(w[0]), "r"(w[1]), "r"(w[2]), "r"(w[3]) : "memory");
+            return;
+        }
         if (ACC) {
             uint32_t prev[3][8];
             #pragma unroll
@@ -544,6 +580,7 @@ __device__ __forceinline__ void epilogue_packed_role(const IgemmParams& p, uint3
                 float sc = 1.f, sh = 0.f;
                 if (oc < p.o) {
                     if (p.dcoef) sc = __ldg(p.dcoef + (long long)tc.n0 * p.o + oc);
+                    if (F8) sc *= weight_scale(p, tc.n0, oc);
                     if (p.bias) sh = __ldg(p.bias + oc);
                 }
                 s_buf[etid] = make_float2(sc * gain, sh * gain);
@@ -558,7 +595,7 @@ __device__ __forceinline__ void epilogue_packed_role(const IgemmParams& p, uint3
         if (t_next < total) { tc_next = decode_tile(p, t_next); nz_next = noise_at(tc_next); }
         const int x = tc.x0 + px, y = tc.y0 + py;
         const bool pix_ok = x < conv_w && y < conv_h && !(p.dbg & 1);
-        __nv_bfloat16* const dst = out + tc.n0 * p.os_n + y * p.os_h + x * p.os_w + tc.col0 + col_begin;
+        ET* const dst = out + tc.n0 * p.os_n + y * p.os_h + x * p.os_w + tc.col0 + col_begin;
         const float2* const s_cs = s_buf + col_begin;
         const int o_left = p.o - (tc.col0 + col_begin);                 // valid columns counted from this warp's first column
         const float nz = nz_raw * gain;
@@ -604,7 +641,7 @@ struct MmaCtx { uint32_t smem_base, b_base, bar_base, tmem_base; };
 // one elected lane issues tcgen05.mma / tcgen05.commit.  PARTS / INNER / KS > 0 are compile-time copies of p.parts /
 // p.inner / (kb / 16) for the common configurations (fully unrolled product / tap / K-step loops, a handful of
 // instructions per MMA); <0, 0, 0> is the generic runtime-bounds version.
-template <int PARTS, int INNER, int KS, bool RES, bool STK = false>
+template <bool F8, int PARTS, int INNER, int KS, bool RES, bool STK = false>
 __device__ __forceinline__ void mma_role(const IgemmParams& p, const MmaCtx mc) {
     const int SA = p.a_stages, SB = p.b_stages;
     auto afull_bar = [&](int s) { return mc.bar_base + 8u * s; };
@@ -616,7 +653,7 @@ __device__ __forceinline__ void mma_role(const IgemmParams& p, const MmaCtx mc) 
     const uint32_t bres_free_bar = mc.bar_base + 8u * (2 * SA + 2 * SB + 4);
     const int parts = PARTS ? PARTS : p.parts;
     const int inner = INNER ? INNER : p.inner;
-    const int k_steps = KS ? KS : p.kb / 16;            // tcgen05.mma kind::f16 has K = 16
+    const int k_steps = KS ? KS : (F8 ? p.kb / 32 : p.kb / 16);     // K per tcgen05.mma: 16 (kind::f16), 32 (kind::f8f6f4) = 32 bytes
     const bool leader = elect_one();
     const bool mma_on = !(p.dbg & 4);
     const uint64_t desc_hi = make_smem_desc(0, p.layout_type, p.sbo_bytes);     // everything but the start address
@@ -660,14 +697,14 @@ __device__ __forceinline__ void mma_role(const IgemmParams& p, const MmaCtx mc) 
                         const uint64_t da0 = desc_hi | (uint64_t)((a16 + j * ky16) & 0x3FFF);
                         const uint64_t da1 = desc_hi | (uint64_t)((a16 + slab16 + j * ky16) & 0x3FFF);
                         if (leader && mma_on) {
-                            umma_bf16(tmem_d, da0, db, p.idesc_stack, acc);
-                            umma_bf16(tmem_d, da0 + 2, db + 2, p.idesc_stack, 1);
-                            umma_bf16(tmem_d, da0 + 4, db + 4, p.idesc_stack, 1);
-                            umma_bf16(tmem_d, da0 + 6, db + 6, p.idesc_stack, 1);
-                            umma_bf16(tmem_d, da1, db, idesc, 1);
-                            umma_bf16(tmem_d, da1 + 2, db + 2, idesc, 1);
-                            umma_bf16(tmem_d, da1 + 4, db + 4, idesc, 1);
-                            umma_bf16(tmem_d, da1 + 6, db + 6, idesc, 1);
+                            umma<F8>(tmem_d, da0, db, p.idesc_stack, acc);
+                            umma<F8>(tmem_d, da0 + 2, db + 2, p.idesc_stack, 1);
+                            umma<F8>(tmem_d, da0 + 4, db + 4, p.idesc_stack, 1);
+                            umma<F8>(tmem_d, da0 + 6, db + 6, p.idesc_stack, 1);
+                            umma<F8>(tmem_d, da1, db, idesc, 1);
+                            umma<F8>(tmem_d, da1 + 2, db + 2, idesc, 1);
+                            umma<F8>(tmem_d, da1 + 4, db + 4, idesc, 1);
+                            umma<F8>(tmem_d, da1 + 6, db + 6, idesc, 1);
                         }
                         acc = 1;
                     }
@@ -692,13 +729,13 @@ __device__ __forceinline__ void mma_role(const IgemmParams& p, const MmaCtx mc) 
                             if (leader && mma_on) {
                                 if (KS == 4) {
                                     // advance 16 elements (32 bytes) along K inside the swizzle row: +2 in the >>4 address field
-                                    umma_bf16(tmem_d, da, db, idesc, acc);
-                                    umma_bf16(tmem_d, da + 2, db + 2, idesc, 1);
-                                    umma_bf16(tmem_d, da + 4, db + 4, idesc, 1);
-                                    umma_bf16(tmem_d, da + 6, db + 6, idesc, 1);
+                                    umma<F8>(tmem_d, da, db, idesc, acc);
+                                    umma<F8>(tmem_d, da + 2, db + 2, idesc, 1);
+                                    umma<F8>(tmem_d, da + 4, db + 4, idesc, 1);
+                                    umma<F8>(tmem_d, da + 6, db + 6, idesc, 1);
                                 } else {
                                     for (int k = 0; k < k_steps; k++)
-                                        umma_bf16(tmem_d, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, acc | (uint32_t)k);
+                                        umma<F8>(tmem_d, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, acc | (uint32_t)k);
                                 }
                             }
                             acc = 1;
@@ -730,7 +767,7 @@ __device__ __forceinline__ void mma_role(const IgemmParams& p, const MmaCtx mc) 
 // (tap_off16) with an 8-row group stride of one slab row (sbo_a) - the tensor core applies the 128-byte swizzle on the absolute
 // shared-memory address, so such views are exact (tools/umma_probe.cu).  Product order: for every part a_pa of the slab, all taps,
 // all weight parts b_pb with pa + pb < parts.  STK: parts == 2 and block_n == 64 -> a0 x [b0; b1] is one N = 128 MMA.
-template <int PARTS, int TAPS, bool STK>
+template <bool F8, int PARTS, int TAPS, bool STK>
 __device__ __forceinline__ void mma_role_slab(const IgemmParams& p, const MmaCtx mc) {
     const int SA = p.a_stages, SB = p.b_stages;
     auto afull_bar = [&](int s) { return mc.bar_base + 8u * s; };
@@ -780,10 +817,10 @@ __device__ __forceinline__ void mma_role_slab(const IgemmParams& p, const MmaCtx
                         const uint64_t db = desc_b_hi | (uint64_t)(b_tap16 & 0x3FFF);
                         const uint32_t id = pa == 0 ? p.idesc_stack : idesc;
                         if (leader && mma_on) {
-                            umma_bf16(tmem_d, da, db, id, acc);
-                            umma_bf16(tmem_d, da + 2, db + 2, id, 1);
-                            umma_bf16(tmem_d, da + 4, db + 4, id, 1);
-                            umma_bf16(tmem_d, da + 6, db + 6, id, 1);
+                            umma<F8>(tmem_d, da, db, id, acc);
+                            umma<F8>(tmem_d, da + 2, db + 2, id, 1);
+                            umma<F8>(tmem_d, da + 4, db + 4, id, 1);
+                            umma<F8>(tmem_d, da + 6, db + 6, id, 1);
                         }
                         acc = 1;
                     } else {
@@ -792,10 +829,10 @@ __device__ __forceinline__ void mma_role_slab(const IgemmParams& p, const MmaCtx
                             if (pa + pb >= parts) break;
                             const uint64_t db = desc_b_hi | (uint64_t)((b_tap16 + pb * bpitch16) & 0x3FFF);
                             if (leader && mma_on) {
-                                umma_bf16(tmem_d, da, db, idesc, acc);
-                                umma_bf16(tmem_d, da + 2, db + 2, idesc, 1);
-                                umma_bf16(tmem_d, da + 4, db + 4, idesc, 1);
-                                umma_bf16(tmem_d, da + 6, db + 6, idesc, 1);
+                                umma<F8>(tmem_d, da, db, idesc, acc);
+                                umma<F8>(tmem_d, da + 2, db + 2, idesc, 1);
+                                umma<F8>(tmem_d, da + 4, db + 4, idesc, 1);
+                                umma<F8>(tmem_d, da + 6, db + 6, idesc, 1);
                             }
                             acc = 1;
                         }
@@ -823,7 +860,7 @@ __device__ __forceinline__ void mma_role_slab(const IgemmParams& p, const MmaCtx
 // r02_igemm64_issuer_ablation.md): with neither activation loads nor epilogue the fp32-parity tile loop runs in 1.23 ms against 1.40 ms for the
 // generic issuer, but the complete kernel stays at 1.57 ms (bf16 mode: 0.83 vs 0.79 ms, uniform-register spills): the issuing warp is not what
 // bounds these layers - the tensor pipe alone, fed from shared memory at N <= 128, already needs 1.23 ms.  Off by default.
-template <int PARTS, bool STK>
+template <bool F8, int PARTS, bool STK>
 __device__ __forceinline__ void mma_role_slab9(const IgemmParams& p, const MmaCtx mc) {
     constexpr int TAPS = 9, PITCH = 10;
     constexpr uint32_t BP16 = 512;          // 64 rows x 128 bytes per weight tile, in 16-byte units
@@ -870,19 +907,19 @@ __device__ __forceinline__ void mma_role_slab9(const IgemmParams& p, const MmaCt
                             // pa == 0: a0 x [b0; b1] (N = 128);  pa == 1: a1 x b0 (N = 64)
                             const uint32_t b_lo = b_lo0 + (uint32_t)(j * PARTS) * BP16;
                             const uint32_t id = pa == 0 ? idesc_stack : idesc;
-                            umma_bf16_lh(tmem_d, a_lo, a_hi, b_lo, b_hi, id, j == 0 ? first : 1u);
-                            umma_bf16_lh(tmem_d, a_lo + 2, a_hi, b_lo + 2, b_hi, id, 1u);
-                            umma_bf16_lh(tmem_d, a_lo + 4, a_hi, b_lo + 4, b_hi, id, 1u);
-                            umma_bf16_lh(tmem_d, a_lo + 6, a_hi, b_lo + 6, b_hi, id, 1u);
+                            umma_lh<F8>(tmem_d, a_lo, a_hi, b_lo, b_hi, id, j == 0 ? first : 1u);
+                            umma_lh<F8>(tmem_d, a_lo + 2, a_hi, b_lo + 2, b_hi, id, 1u);
+                            umma_lh<F8>(tmem_d, a_lo + 4, a_hi, b_lo + 4, b_hi, id, 1u);
+                            umma_lh<F8>(tmem_d, a_lo + 6, a_hi, b_lo + 6, b_hi, id, 1u);
                         } else {
                             #pragma unroll
                             for (int pb = 0; pb < PARTS; pb++) {
                                 if (pa + pb >= PARTS) break;
                                 const uint32_t b_lo = b_lo0 + (uint32_t)(j * PARTS + pb) * BP16;
-                                umma_bf16_lh(tmem_d, a_lo, a_hi, b_lo, b_hi, idesc, (j == 0 && pb == 0) ? first : 1u);
-                                umma_bf16_lh(tmem_d, a_lo + 2, a_hi, b_lo + 2, b_hi, idesc, 1u);
-                                umma_bf16_lh(tmem_d, a_lo + 4, a_hi, b_lo + 4, b_hi, idesc, 1u);
-                                umma_bf16_lh(tmem_d, a_lo + 6, a_hi, b_lo + 6, b_hi, idesc, 1u);
+                                umma_lh<F8>(tmem_d, a_lo, a_hi, b_lo, b_hi, idesc, (j == 0 && pb == 0) ? first : 1u);
+                                umma_lh<F8>(tmem_d, a_lo + 2, a_hi, b_lo + 2, b_hi, idesc, 1u);
+                                umma_lh<F8>(tmem_d, a_lo + 4, a_hi, b_lo + 4, b_hi, idesc, 1u);
+                                umma_lh<F8>(tmem_d, a_lo + 6, a_hi, b_lo + 6, b_hi, idesc, 1u);
                             }
                         }
                     }
@@ -902,8 +939,9 @@ __device__ __forceinline__ void mma_role_slab9(const IgemmParams& p, const MmaCt
     __syncwarp();
 }
 
-// EPI 0: every epilogue option;  EPI 1: the lean operand-format epilogue only (epilogue_packed_role; smaller code and register footprint)
-template <int EPI>
+// EPI 0: every epilogue option;  EPI 1: the lean operand-format epilogue only (epilogue_packed_role; smaller code and register footprint).
+// F8: e4m3 operands (kind::f8f6f4; channel blocks of kb bytes = kb channels), weight column scales in the epilogue; EPI 1 writes e4m3.
+template <int EPI, bool F8>
 __global__ void __launch_bounds__(kThreads, 1)
 igemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, const IgemmParams p) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -1021,31 +1059,40 @@ igemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
     } else if (warp == 1) {
         // ===================== MMA issuer =====================
         const MmaCtx mc{smem_base, b_base, bar_base, tmem_base};
-        const int ks = p.kb == 64 ? 4 : 0;
+        const int ks = p.kb == (F8 ? 128 : 64) ? 4 : 0;     // 128-byte channel blocks
         const bool res = p.b_resident != 0;
-        if (p.reuse == 2 && p.slab9) {
-            if (p.parts == 1) mma_role_slab9<1, false>(p, mc);
-            else if (p.stack) mma_role_slab9<2, true>(p, mc);
-            else mma_role_slab9<2, false>(p, mc);
+        if constexpr (F8) {     // e4m3 operands are one part
+            if (p.reuse == 2 && p.slab9) mma_role_slab9<F8, 1, false>(p, mc);
+            else if (p.reuse == 2) { if (p.inner == 9) mma_role_slab<F8, 1, 9, false>(p, mc); else mma_role_slab<F8, 1, 0, false>(p, mc); }
+            else if (ks == 4 && p.inner == 3) { if (res) mma_role<F8, 1, 3, 4, true>(p, mc); else mma_role<F8, 1, 3, 4, false>(p, mc); }
+            else if (ks == 4 && p.inner == 7) mma_role<F8, 1, 7, 4, false>(p, mc);
+            else if (ks == 4 && p.inner == 1) { if (res) mma_role<F8, 1, 1, 4, true>(p, mc); else mma_role<F8, 1, 1, 4, false>(p, mc); }
+            else if (res) mma_role<F8, 1, 0, 0, true>(p, mc);
+            else mma_role<F8, 1, 0, 0, false>(p, mc);
+        }
+        else if (p.reuse == 2 && p.slab9) {
+            if (p.parts == 1) mma_role_slab9<F8, 1, false>(p, mc);
+            else if (p.stack) mma_role_slab9<F8, 2, true>(p, mc);
+            else mma_role_slab9<F8, 2, false>(p, mc);
         }
         else if (p.reuse == 2) {
-            if (p.inner == 9 && p.parts == 1) mma_role_slab<1, 9, false>(p, mc);
-            else if (p.inner == 9 && p.parts == 2 && p.stack) mma_role_slab<2, 9, true>(p, mc);
-            else if (p.inner == 9 && p.parts == 2) mma_role_slab<2, 9, false>(p, mc);
-            else if (p.stack) mma_role_slab<2, 0, true>(p, mc);
-            else mma_role_slab<0, 0, false>(p, mc);
+            if (p.inner == 9 && p.parts == 1) mma_role_slab<F8, 1, 9, false>(p, mc);
+            else if (p.inner == 9 && p.parts == 2 && p.stack) mma_role_slab<F8, 2, 9, true>(p, mc);
+            else if (p.inner == 9 && p.parts == 2) mma_role_slab<F8, 2, 9, false>(p, mc);
+            else if (p.stack) mma_role_slab<F8, 2, 0, true>(p, mc);
+            else mma_role_slab<F8, 0, 0, false>(p, mc);
         }
-        else if (ks == 4 && p.inner == 3 && p.parts == 1) { if (res) mma_role<1, 3, 4, true>(p, mc); else mma_role<1, 3, 4, false>(p, mc); }
-        else if (ks == 4 && p.inner == 3 && p.parts == 2 && p.stack) mma_role<2, 3, 4, true, true>(p, mc);
-        else if (ks == 4 && p.inner == 1 && p.parts == 2 && p.stack) mma_role<2, 1, 4, true, true>(p, mc);
-        else if (ks == 4 && p.inner == 3 && p.parts == 2) { if (res) mma_role<2, 3, 4, true>(p, mc); else mma_role<2, 3, 4, false>(p, mc); }
-        else if (ks == 4 && p.inner == 3 && p.parts == 3) mma_role<3, 3, 4, false>(p, mc);
-        else if (ks == 4 && p.inner == 7 && p.parts == 1) mma_role<1, 7, 4, false>(p, mc);
-        else if (ks == 4 && p.inner == 7 && p.parts == 2) mma_role<2, 7, 4, false>(p, mc);
-        else if (ks == 4 && p.inner == 1 && p.parts == 1) { if (res) mma_role<1, 1, 4, true>(p, mc); else mma_role<1, 1, 4, false>(p, mc); }
-        else if (ks == 4 && p.inner == 1 && p.parts == 2) { if (res) mma_role<2, 1, 4, true>(p, mc); else mma_role<2, 1, 4, false>(p, mc); }
-        else if (res) mma_role<0, 0, 0, true>(p, mc);
-        else mma_role<0, 0, 0, false>(p, mc);
+        else if (ks == 4 && p.inner == 3 && p.parts == 1) { if (res) mma_role<F8, 1, 3, 4, true>(p, mc); else mma_role<F8, 1, 3, 4, false>(p, mc); }
+        else if (ks == 4 && p.inner == 3 && p.parts == 2 && p.stack) mma_role<F8, 2, 3, 4, true, true>(p, mc);
+        else if (ks == 4 && p.inner == 1 && p.parts == 2 && p.stack) mma_role<F8, 2, 1, 4, true, true>(p, mc);
+        else if (ks == 4 && p.inner == 3 && p.parts == 2) { if (res) mma_role<F8, 2, 3, 4, true>(p, mc); else mma_role<F8, 2, 3, 4, false>(p, mc); }
+        else if (ks == 4 && p.inner == 3 && p.parts == 3) mma_role<F8, 3, 3, 4, false>(p, mc);
+        else if (ks == 4 && p.inner == 7 && p.parts == 1) mma_role<F8, 1, 7, 4, false>(p, mc);
+        else if (ks == 4 && p.inner == 7 && p.parts == 2) mma_role<F8, 2, 7, 4, false>(p, mc);
+        else if (ks == 4 && p.inner == 1 && p.parts == 1) { if (res) mma_role<F8, 1, 1, 4, true>(p, mc); else mma_role<F8, 1, 1, 4, false>(p, mc); }
+        else if (ks == 4 && p.inner == 1 && p.parts == 2) { if (res) mma_role<F8, 2, 1, 4, true>(p, mc); else mma_role<F8, 2, 1, 4, false>(p, mc); }
+        else if (res) mma_role<F8, 0, 0, 0, true>(p, mc);
+        else mma_role<F8, 0, 0, 0, false>(p, mc);
     } else if (EPI == 1) {
         // ===================== epilogue warps, operand-format hand-over =====================
 #define PGPP_PACKED(ACT) \
@@ -1053,9 +1100,19 @@ igemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
                             else         epilogue_packed_role<ACT, false, true>(p, bar_base, tmem_base, s_params, warp, lane); } \
         else              { if (p.stack) epilogue_packed_role<ACT, true, false>(p, bar_base, tmem_base, s_params, warp, lane);  \
                             else         epilogue_packed_role<ACT, false, false>(p, bar_base, tmem_base, s_params, warp, lane); }
+#define PGPP_PACKED_F8(ACT) \
+        if (p.accumulate) epilogue_packed_role<ACT, false, true, true>(p, bar_base, tmem_base, s_params, warp, lane);  \
+        else              epilogue_packed_role<ACT, false, false, true>(p, bar_base, tmem_base, s_params, warp, lane);
+        if constexpr (F8) {     // one part: never stacked
+            if (p.act_fn == PGPP_ACT_LINEAR) { PGPP_PACKED_F8(PGPP_ACT_LINEAR) }
+            else if (p.act_fn == PGPP_ACT_RELU) { PGPP_PACKED_F8(PGPP_ACT_RELU) }
+            else { PGPP_PACKED_F8(PGPP_ACT_LRELU) }
+        } else {
         if (p.act_fn == PGPP_ACT_LINEAR) { PGPP_PACKED(PGPP_ACT_LINEAR) }
         else if (p.act_fn == PGPP_ACT_RELU) { PGPP_PACKED(PGPP_ACT_RELU) }
         else { PGPP_PACKED(PGPP_ACT_LRELU) }
+        }
+#undef PGPP_PACKED_F8
 #undef PGPP_PACKED
     } else {
         // ===================== epilogue warps =====================
@@ -1088,6 +1145,7 @@ igemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
                         float sc = 1.f, sh = 0.f;
                         if (oc < p.o && phase < p.phases) {
                             if (p.dcoef) sc = __ldg(p.dcoef + (long long)tc.n0 * p.o + oc);
+                            if (F8) sc *= weight_scale(p, tc.n0, g);
                             if (p.bias) sh = __ldg(p.bias + oc);
                         }
                         if (p.spade_x) {        // (rstd | mean of the normalised tensor, bias of gamma | beta)
@@ -1114,10 +1172,10 @@ igemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
             // instance-norm partials: row (pixel tile, lane quarter) of the workspace, pixel tiles numbered sample-major
             float* stats_row = nullptr;
             if (p.stats_ws) stats_row = p.stats_ws + ((long long)fast_div((unsigned)t, p.div_col_m, p.div_col_s) * 4 + quarter) * p.o;
-            if (p.spade_x) epilogue_spade(p, tc, tmem_tile, pc, half, s_cs);
-            else if (p.out_dtype == PGPP_F32) epilogue_dispatch<float>(p, tc, tmem_tile, pc, col_begin, col_end, s_cs, fast, nz_pre, stats_row);
-            else if (p.out_dtype == PGPP_BF16) epilogue_dispatch<__nv_bfloat16>(p, tc, tmem_tile, pc, col_begin, col_end, s_cs, fast, nz_pre, nullptr);
-            else epilogue_dispatch<__half>(p, tc, tmem_tile, pc, col_begin, col_end, s_cs, fast, nz_pre, nullptr);
+            if (p.spade_x) epilogue_spade<F8>(p, tc, tmem_tile, pc, half, s_cs);
+            else if (p.out_dtype == PGPP_F32) epilogue_dispatch<float, F8>(p, tc, tmem_tile, pc, col_begin, col_end, s_cs, fast, nz_pre, stats_row);
+            else if (p.out_dtype == PGPP_BF16) epilogue_dispatch<__nv_bfloat16, F8>(p, tc, tmem_tile, pc, col_begin, col_end, s_cs, fast, nz_pre, nullptr);
+            else epilogue_dispatch<__half, F8>(p, tc, tmem_tile, pc, col_begin, col_end, s_cs, fast, nz_pre, nullptr);
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(tempty_bar(buf));
@@ -1233,7 +1291,15 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
     PGPP_REQUIRE(d->products == 1 || d->products == 3 || d->products == 6, "products must be 1, 3 or 6");
     const int need_parts = d->products == 1 ? 1 : (d->products == 3 ? 2 : 3);
     PGPP_REQUIRE(d->a_parts >= need_parts && d->b_parts >= need_parts, "operand parts do not cover the requested products");
-    PGPP_REQUIRE(d->out_dtype == PGPP_F32 || d->out_dtype == PGPP_BF16 || d->out_dtype == PGPP_F16, "unsupported output dtype");
+    const bool e4m3 = d->operand_e4m3 != 0;
+    const int esize = e4m3 ? 1 : 2;             // bytes per operand element
+    PGPP_REQUIRE(d->out_dtype == PGPP_F32 || d->out_dtype == PGPP_BF16 || d->out_dtype == PGPP_F16 || (e4m3 && d->out_dtype == PGPP_E4M3),
+                 "unsupported output dtype (e4m3 output needs e4m3 operands)");
+    if (e4m3) {
+        PGPP_REQUIRE(d->products == 1 && !d->operand_f16, "e4m3 operands are one part (products must be 1)");
+        PGPP_REQUIRE(d->wscale != nullptr, "e4m3 operands need the weight column scales (wscale)");
+        PGPP_REQUIRE(d->c_pad % 32 == 0, "e4m3 operands: c_pad must be a multiple of 32");
+    }
     PGPP_REQUIRE(d->act_fn >= 1 && d->act_fn <= 9, "no CUDA kernel found for the specified activation func");
     PGPP_REQUIRE(((uintptr_t)d->act & 15) == 0 && ((uintptr_t)d->wgt & 15) == 0, "packed operands must be 16-byte aligned");
     const int out_parts = d->out_parts <= 0 ? 1 : d->out_parts;
@@ -1242,7 +1308,7 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
                                     d->out_stride[3] % 8 == 0 && d->out_part_stride % 8 == 0 && ((uintptr_t)d->out & 15) == 0),
                  "split output needs bf16, channels-innermost, 16-byte aligned pixels, out channels % 16 == 0");
     const int pix_stride = d->act_pixel_stride > 0 ? d->act_pixel_stride : d->c_pad;
-    PGPP_REQUIRE(pix_stride >= d->c_pad && pix_stride % 8 == 0, "act_pixel_stride must be >= c_pad and a multiple of 8");
+    PGPP_REQUIRE(pix_stride >= d->c_pad && (pix_stride * esize) % 16 == 0, "act_pixel_stride must be >= c_pad and a multiple of 16 bytes");
     const int up = d->phases == 4 ? 2 : 1;
     PGPP_REQUIRE(d->out_h == d->conv_h * up && d->out_w == d->conv_w * up, "output size does not match the conv grid");
 
@@ -1252,7 +1318,8 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
     IgemmParams p;
     p.n = d->n; p.h = d->h; p.w = d->w; p.conv_h = d->conv_h; p.conv_w = d->conv_w;
     p.kh = d->kh; p.kw = d->kw; p.pad_y = d->pad_y; p.pad_x = d->pad_x; p.stride = d->stride;
-    p.kb = (d->c_pad % 64 == 0) ? 64 : ((d->c_pad % 32 == 0) ? 32 : 16);
+    if (e4m3) p.kb = (d->c_pad % 128 == 0) ? 128 : ((d->c_pad % 64 == 0) ? 64 : 32);      // channels = bytes
+    else p.kb = (d->c_pad % 64 == 0) ? 64 : ((d->c_pad % 32 == 0) ? 32 : 16);
     p.num_cb = d->c_pad / p.kb;
     p.parts = need_parts;
     // products of the bf16 expansions: parts 1 -> a0b0; 2 -> a0b0 + a1b0 + a0b1; 3 -> + a2b0 + a1b1 + a0b2
@@ -1272,12 +1339,13 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
     // filter-column slabs; an 8 x 16 pixel tile reads ONE (8 + kw - 1) x (16 + kh - 1) slab per (channel block, part) instead and
     // takes every tap as a row-shifted descriptor view of it (2.7x fewer activation bytes for 3 x 3).  Needs resident weights.
     const int slab_pitch = 8 + d->kw - 1, slab_rows2 = 16 + d->kh - 1;
-    const bool slab2_shape = d->stride == 1 && d->kh * d->kw > 1 && d->kh * d->kw <= 64 && dil_y == 1 && d->c_pad % 64 == 0 && d->block_n <= 64 &&
+    const int row_ch = e4m3 ? 128 : 64;         // channels of a 128-byte row
+    const bool slab2_shape = d->stride == 1 && d->kh * d->kw > 1 && d->kh * d->kw <= 64 && dil_y == 1 && d->c_pad % row_ch == 0 && d->block_n <= 64 &&
                              d->phases * d->phase_stride <= d->block_n && d->conv_w >= 8 && d->conv_h >= 16 && need_parts <= 2 &&
                              !env.igemm_no_slab2 && !env.igemm_no_resident;
     if (slab2_shape) {
         const long long stage = ((long long)slab_pitch * slab_rows2 * 128 + 1023) & ~1023ll;
-        const long long n_bt = (long long)(d->c_pad / 64) * d->kh * d->kw * need_parts;
+        const long long n_bt = (long long)(d->c_pad / row_ch) * d->kh * d->kw * need_parts;
         const long long b_pitch2 = ((long long)d->block_n * 128 + 1023) & ~1023ll;
         const long long need = 1024 + 2 * stage + n_bt * b_pitch2 + 8 * (2 * 2 + 2 * n_bt + 5) + 32 + 16ll * d->block_n;
         const long long tiles = (long long)((d->conv_w + 7) / 8) * ((d->conv_h + 15) / 16) * d->n;
@@ -1297,7 +1365,7 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
     p.tiles_n = (d->n + p.tn - 1) / p.tn;
     p.tiles_col = (d->phases * d->phase_stride + d->block_n - 1) / d->block_n;
     p.total_tiles = (long long)p.tiles_x * p.tiles_y * p.tiles_n * p.tiles_col;
-    const unsigned row_bytes = (unsigned)p.kb * 2;
+    const unsigned row_bytes = (unsigned)(p.kb * esize);
     const int slab_rows = p.tn * (p.th + (p.inner - 1) * dil_y) * p.tw;        // multiple of 8 (TW % 8 == 0 with reuse, 128 without)
     p.slab_bytes = (unsigned)slab_rows * row_bytes;
     p.a_tx_bytes = p.parts * p.slab_bytes;
@@ -1320,7 +1388,8 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
     p.sbo_bytes = 8 * row_bytes;
     // instruction descriptor (cute/arch/mma_sm100_desc.hpp InstrDescriptor): fp32 accum, bf16 A/B, K-major, M = 128
     // a_format / b_format (bits 7-9 / 10-12): 1 = bf16, 0 = f16 (the fp16 layers of the discriminator run native f16 MMAs)
-    const unsigned ab_fmt = d->operand_f16 ? 0u : ((1u << 7) | (1u << 10));
+    // kind::f8f6f4: a_format / b_format 0 = E4M3
+    const unsigned ab_fmt = (d->operand_f16 || e4m3) ? 0u : ((1u << 7) | (1u << 10));
     PGPP_REQUIRE(!d->operand_f16 || d->products == 1, "fp16 operands are a single part (products must be 1)");
     p.idesc = (1u << 4) | ab_fmt | ((unsigned)(d->block_n >> 3) << 17) | ((unsigned)(kTileM >> 4) << 24);
     unsigned cols = (unsigned)pow2_ceil(2 * d->block_n); if (cols < 32) cols = 32;
@@ -1361,9 +1430,9 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
         PGPP_REQUIRE(d->spade_mean && d->spade_rstd, "SPADE epilogue needs mean and rstd");
         PGPP_REQUIRE(d->phases == 1 && d->o % 32 == 0 && d->block_n == d->o && d->stride == 1 && p.tn == 1,
                      "SPADE epilogue: o = 2C (gamma | beta) with C % 16 == 0 in ONE column tile (block_n == o), stride 1, images of at least 128 pixels");
-        PGPP_REQUIRE(d->out_dtype == PGPP_BF16 && d->out_stride[1] == 1 && !d->accumulate && d->out_stride[3] % 8 == 0 &&
-                     d->out_part_stride % 8 == 0 && ((uintptr_t)d->out & 15) == 0,
-                     "SPADE epilogue writes the channels-innermost bf16 operand format (16-byte aligned pixels)");
+        PGPP_REQUIRE((d->out_dtype == PGPP_BF16 || (e4m3 && d->out_dtype == PGPP_E4M3 && out_parts == 1 && d->out_stride[3] % 16 == 0)) &&
+                     d->out_stride[1] == 1 && !d->accumulate && d->out_stride[3] % 8 == 0 && d->out_part_stride % 8 == 0 && ((uintptr_t)d->out & 15) == 0,
+                     "SPADE epilogue writes the channels-innermost bf16 (or, from e4m3 operands, e4m3) operand format (16-byte aligned pixels)");
         PGPP_REQUIRE(d->act_fn == PGPP_ACT_LINEAR && d->gain == 1.f && d->clamp < 0.f && !d->noise && !d->dcoef,
                      "SPADE epilogue: the GEMM itself must be linear (no noise, demodulation, gain or clamp)");
     }
@@ -1372,7 +1441,7 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
     // stacked products (see mma_role): fp32-parity mode with 2 parts, resident 64-column weight tiles, fast epilogue
     p.stack = (need_parts == 2 && d->block_n == 64 && p.b_resident && p.kb == 64 && (p.inner == 3 || p.inner == 1 || p.reuse == 2) && p.tn == 1 && p.fold_gain &&
                !d->spade_x && !env.igemm_no_stack) ? 1 : 0;
-    p.slab9 = (p.reuse == 2 && d->kh == 3 && d->kw == 3 && p.kb == 64 && d->block_n == 64 && p.b_pitch == 8192 && need_parts <= 2 &&
+    p.slab9 = (p.reuse == 2 && d->kh == 3 && d->kw == 3 && row_bytes == 128 && d->block_n == 64 && p.b_pitch == 8192 && need_parts <= 2 &&
                env.igemm_slab9) ? 1 : 0;       // opt-in (PGPP_IGEMM_SLAB9=1): measured neutral in fp32-parity mode, 5 % slower in bf16 mode
     p.acc_cols = p.stack ? 2 * d->block_n : d->block_n;
     p.idesc_stack = (1u << 4) | ab_fmt | ((unsigned)((2 * d->block_n) >> 3) << 17) | ((unsigned)(kTileM >> 4) << 24);
@@ -1386,6 +1455,7 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
     magic((unsigned)p.tiles_y, p.div_y_m, p.div_y_s);
     PGPP_REQUIRE(p.total_tiles < (1ll << 31), "too many tiles");
     p.dbg = env.igemm_debug;
+    p.wscale = e4m3 ? d->wscale : nullptr;
 
     // instance-norm partials of the output (pgpp_conv_desc.stats_ws): fast float32 NCHW epilogue, full pixel tiles, whole 16-column chunks
     const bool stats_ok = p.tn == 1 && p.fold_gain && d->out_dtype == PGPP_F32 && d->phases == 1 && !d->accumulate && !d->spade_x && d->o % 16 == 0 &&
@@ -1400,36 +1470,44 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
     CUtensorMap map_a, map_b;
     {
         const cuuint64_t dims[5] = {(cuuint64_t)d->c_pad, (cuuint64_t)d->w, (cuuint64_t)d->h, (cuuint64_t)d->n, (cuuint64_t)d->a_parts};
-        const cuuint64_t strides[4] = {(cuuint64_t)pix_stride * 2, (cuuint64_t)pix_stride * 2 * d->w, (cuuint64_t)pix_stride * 2 * d->w * d->h,
-                                       (cuuint64_t)pix_stride * 2 * d->w * d->h * d->n};
+        const cuuint64_t pb = (cuuint64_t)pix_stride * esize;
+        const cuuint64_t strides[4] = {pb, pb * d->w, pb * d->w * d->h, pb * d->w * d->h * d->n};
         cuuint32_t box[5] = {(cuuint32_t)p.kb, (cuuint32_t)(p.tw * d->stride), (cuuint32_t)((p.th + (p.inner - 1) * dil_y) * d->stride), (cuuint32_t)p.tn, 1};
         if (p.reuse == 2) { box[1] = (cuuint32_t)slab_pitch; box[2] = (cuuint32_t)slab_rows2; }
         const cuuint32_t estr[5] = {1, (cuuint32_t)d->stride, (cuuint32_t)d->stride, 1, 1};
         const CUtensorMapSwizzle sw = row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (row_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
-        CUresult r = encode(&map_a, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(d->act), dims, strides, box, estr,
+        const CUtensorMapDataType el = e4m3 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+        CUresult r = encode(&map_a, el, 5, const_cast<void*>(d->act), dims, strides, box, estr,
                             CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(activations) failed with CUresult %d", (int)r); return PGPP_ERR_CUDA; }
         const cuuint64_t wrows = (cuuint64_t)d->o_rows * d->kh * d->kw;
         const cuuint64_t wdims[4] = {(cuuint64_t)d->c_pad, wrows, (cuuint64_t)d->b_parts, (cuuint64_t)(d->wgt_per_sample ? d->n : 1)};
-        const cuuint64_t wstrides[3] = {(cuuint64_t)d->c_pad * 2, (cuuint64_t)d->c_pad * 2 * wrows, (cuuint64_t)d->c_pad * 2 * wrows * d->b_parts};
+        const cuuint64_t rb = (cuuint64_t)d->c_pad * esize;
+        const cuuint64_t wstrides[3] = {rb, rb * wrows, rb * wrows * d->b_parts};
         const cuuint32_t wbox[4] = {(cuuint32_t)p.kb, (cuuint32_t)d->block_n, 1, 1};
         const cuuint32_t westr[4] = {1, 1, 1, 1};
-        r = encode(&map_b, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(d->wgt), wdims, wstrides, wbox, westr,
+        r = encode(&map_b, el, 4, const_cast<void*>(d->wgt), wdims, wstrides, wbox, westr,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(weights) failed with CUresult %d", (int)r); return PGPP_ERR_CUDA; }
     }
     // lean operand-format epilogue (EPI 1) when the launch needs nothing else
-    const bool epi_packed = p.tn == 1 && p.fold_gain && d->out_dtype == PGPP_BF16 && p.os_c == 1 && d->phases == 1 && !d->spade_x &&
-                            d->o % 16 == 0 && d->block_n >= 32 && ((uintptr_t)d->out & 31) == 0 && p.os_w % 16 == 0 && p.os_h % 16 == 0 &&
-                            p.os_n % 16 == 0 && p.out_part_stride % 16 == 0 && !env.igemm_no_lean_epilogue;
+    // (e4m3 operands: the lean epilogue writes e4m3 - and is the only one that does)
+    const bool epi_packed = p.tn == 1 && p.fold_gain && d->out_dtype == (e4m3 ? PGPP_E4M3 : PGPP_BF16) && p.os_c == 1 && d->phases == 1 && !d->spade_x &&
+                            d->o % 16 == 0 && d->block_n >= 32 && ((uintptr_t)d->out & (e4m3 ? 15 : 31)) == 0 && p.os_w % 16 == 0 && p.os_h % 16 == 0 &&
+                            p.os_n % 16 == 0 && p.out_part_stride % 16 == 0 && (!env.igemm_no_lean_epilogue || e4m3);
+    PGPP_REQUIRE(d->out_dtype != PGPP_E4M3 || d->spade_x || (epi_packed && out_parts == 1 && !d->stats_ws),
+                 "e4m3 output: one part, channels-innermost, 16-byte aligned pixels, o % 16 == 0, phases == 1, one sample per tile, "
+                 "linear / relu / lrelu with gain > 0, block_n >= 32");
     {
         // once per device (the attribute is per function per context)
         static std::atomic<bool> done[64];
         int dev = 0;
         cudaGetDevice(&dev);
         if (dev < 0 || dev >= 64 || !done[dev].load(std::memory_order_acquire)) {
-            PGPP_CUDA_OK(cudaFuncSetAttribute(igemm_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-            PGPP_CUDA_OK(cudaFuncSetAttribute(igemm_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+            PGPP_CUDA_OK(cudaFuncSetAttribute(igemm_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+            PGPP_CUDA_OK(cudaFuncSetAttribute(igemm_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+            PGPP_CUDA_OK(cudaFuncSetAttribute(igemm_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+            PGPP_CUDA_OK(cudaFuncSetAttribute(igemm_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
             if (dev >= 0 && dev < 64) done[dev].store(true, std::memory_order_release);
         }
     }
@@ -1439,8 +1517,11 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
     PGPP_REQUIRE(epi_packed || out_parts == 1 || !d->accumulate,
                  "accumulating into a split (operand-format) output needs the lean epilogue: one sample per tile, linear / relu / lrelu with gain > 0, "
                  "32-byte aligned pixels, block_n >= 32, phases == 1");
-    if (epi_packed) igemm_kernel<1><<<(unsigned)grid, kThreads, smem_bytes, (cudaStream_t)stream>>>(map_a, map_b, p);
-    else igemm_kernel<0><<<(unsigned)grid, kThreads, smem_bytes, (cudaStream_t)stream>>>(map_a, map_b, p);
+    if (e4m3) {
+        if (epi_packed) igemm_kernel<1, true><<<(unsigned)grid, kThreads, smem_bytes, (cudaStream_t)stream>>>(map_a, map_b, p);
+        else igemm_kernel<0, true><<<(unsigned)grid, kThreads, smem_bytes, (cudaStream_t)stream>>>(map_a, map_b, p);
+    } else if (epi_packed) igemm_kernel<1, false><<<(unsigned)grid, kThreads, smem_bytes, (cudaStream_t)stream>>>(map_a, map_b, p);
+    else igemm_kernel<0, false><<<(unsigned)grid, kThreads, smem_bytes, (cudaStream_t)stream>>>(map_a, map_b, p);
     count_launch();
     PGPP_CUDA_OK(cudaGetLastError());
     return PGPP_OK;

@@ -13,6 +13,7 @@ struct PackArgs {
     long long s_n, s_c, s_h, s_w;
     long long part_stride;      // elements between parts = n*h*w*c_pad
     int f16;                    // 1: the operand is IEEE half (one part) instead of the bf16 expansion (fp16 layers, native f16 MMA)
+    int e4m3;                   // 1: the operand is ONE part of e4m3 bytes (fp8 inference precision); out and the strides count bytes
     // gradient of a fused bias_act (pgpp_pack_act_gradient): x = dy, gate = the saved output y (same dtype and strides)
     const void* gate; int act; float alpha, gain, clamp;
     float* csum;                // [N][C][x_tiles * y_tiles] per-tile channel sums of the packed gradient (the bias gradient), or NULL
@@ -40,7 +41,9 @@ struct TileGeom { int log_tw, x_tiles, y_tiles, c_tiles; };
 
 // 8 consecutive channels of pixel k as one 16-byte packet of the current bf16 part; `more`: another part follows, so the residual
 // v - bf16(v) is left in v (packed conversions: one cvt.rn.bf16x2.f32 per channel pair)
-__device__ __forceinline__ uint4 split_packet(float (&v)[8][4], int k, int f16 = 0, bool more = true) {
+__device__ __forceinline__ uint4 split_packet(float (&v)[8][4], int k, int f16 = 0, bool more = true, int e4m3 = 0) {
+    if (e4m3)       // 8 bytes in the low half of the packet
+        return make_uint4(e4m3x4(v[0][k], v[1][k], v[2][k], v[3][k]), e4m3x4(v[4][k], v[5][k], v[6][k], v[7][k]), 0u, 0u);
     if (f16) {
         __align__(16) __half hq[8];
         #pragma unroll
@@ -63,12 +66,12 @@ __device__ __forceinline__ uint4 split_packet(float (&v)[8][4], int k, int f16 =
 // writes the tile held in v (see above) to out[part][n][y][x][c_off + c0 ...]; sm = parts * 128 * 8 packets
 __device__ __forceinline__ void emit_tile(float (&v)[8][4], uint4* sm, int parts, __nv_bfloat16* out, long long part_stride,
                                           int n, int h, int w, int y0, int x0, int log_tw, int c0, int c_lim, int c_total, int c_off,
-                                          int f16 = 0) {
+                                          int f16 = 0, int e4m3 = 0) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     for (int part = 0; part < parts; part++) {
         #pragma unroll
         for (int k = 0; k < 4; k++)
-            sm[(part * 128 + 4 * lane + k) * 8 + (warp ^ (lane & 7))] = split_packet(v, k, f16, part + 1 < parts);
+            sm[(part * 128 + 4 * lane + k) * 8 + (warp ^ (lane & 7))] = split_packet(v, k, f16, part + 1 < parts, e4m3);
     }
     __syncthreads();
     const int tw_mask = (1 << log_tw) - 1;
@@ -79,8 +82,10 @@ __device__ __forceinline__ void emit_tile(float (&v)[8][4], uint4* sm, int parts
             const int px = item >> 3, ch = item & 7;
             const int y = y0 + (px >> log_tw), x = x0 + (px & tw_mask);
             if (y < h && x < w && c0 + ch * 8 < c_lim) {
-                __nv_bfloat16* dst = out + part * part_stride + (((long long)n * h + y) * w + x) * c_total + c_off + c0 + ch * 8;
-                *reinterpret_cast<uint4*>(dst) = sm[(part * 128 + px) * 8 + (ch ^ ((px >> 2) & 7))];
+                const long long idx = part * part_stride + (((long long)n * h + y) * w + x) * c_total + c_off + c0 + ch * 8;
+                const uint4 pk = sm[(part * 128 + px) * 8 + (ch ^ ((px >> 2) & 7))];
+                if (e4m3) *reinterpret_cast<uint2*>(reinterpret_cast<uint8_t*>(out) + idx) = make_uint2(pk.x, pk.y);
+                else *reinterpret_cast<uint4*>(out + idx) = pk;
             }
         }
     }
@@ -247,7 +252,7 @@ __global__ void __launch_bounds__(256) pack_nchw_kernel(PackArgs p, TileGeom g) 
                 p.csum[((long long)n * p.c + c) * ((long long)g.x_tiles * g.y_tiles) + (long long)yt * g.x_tiles + xt] = s1;
         }
     }
-    emit_tile(v, sm_packets, p.parts, p.out, p.part_stride, n, p.h, p.w, y0, x0, g.log_tw, c0, p.c_pad, p.c_total, p.c_off, p.f16);
+    emit_tile(v, sm_packets, p.parts, p.out, p.part_stride, n, p.h, p.w, y0, x0, g.log_tw, c0, p.c_pad, p.c_total, p.c_off, p.f16, p.e4m3);
 }
 
 // any strides (channels_last inputs are coalesced here): one thread per (pixel, channel)
@@ -264,7 +269,9 @@ __global__ void __launch_bounds__(256) pack_generic_kernel(PackArgs p, long long
             v = (float)to_acc<T>(((const T*)p.x)[n * p.s_n + c * p.s_c + y * p.s_h + x * p.s_w]);
             if (p.scale) v *= p.scale[n * p.c + c];
         }
-        split_store(v, p.out + (e / p.c_pad) * p.c_total + p.c_off + c, p.part_stride, p.parts, p.f16);
+        const long long idx = (e / p.c_pad) * p.c_total + p.c_off + c;
+        if (p.e4m3) reinterpret_cast<uint8_t*>(p.out)[idx] = (uint8_t)__nv_cvt_float_to_fp8(v, __NV_SATFINITE, __NV_E4M3);
+        else split_store(v, p.out + idx, p.part_stride, p.parts, p.f16);
     }
 }
 
@@ -757,7 +764,7 @@ extern "C" int pgpp_modulate_weights(const float* master, const float* s, void* 
 namespace pgpp {
 struct PackGate { const void* y; int act; float alpha, gain, clamp; float* csum; };
 static int pack_slice(const void* x, const int64_t size[4], const int64_t stride[4], int dtype, const float* scale, void* out,
-                      int c_pad, int c_total, int c_off, int parts, int f16, void* stream, const PackGate* gate = nullptr);
+                      int c_pad, int c_total, int c_off, int parts, int f16, void* stream, const PackGate* gate = nullptr, int e4m3 = 0);
 }
 
 extern "C" int pgpp_pack_act_gradient_tiles(int h, int w) {
@@ -789,8 +796,13 @@ extern "C" int pgpp_pack_activations_f16(const void* x, const int64_t size[4], c
     return pgpp::pack_slice(x, size, stride, dtype, scale, out, c_pad, c_total, c_off, 1, 1, stream);
 }
 
+extern "C" int pgpp_pack_activations_e4m3(const void* x, const int64_t size[4], const int64_t stride[4], int dtype,
+                                          const float* scale, void* out, int c_pad, int c_total, int c_off, void* stream) {
+    return pgpp::pack_slice(x, size, stride, dtype, scale, out, c_pad, c_total, c_off, 1, 0, stream, nullptr, 1);
+}
+
 int pgpp::pack_slice(const void* x, const int64_t size[4], const int64_t stride[4], int dtype, const float* scale, void* out,
-                     int c_pad, int c_total, int c_off, int parts, int f16, void* stream, const PackGate* gate) {
+                     int c_pad, int c_total, int c_off, int parts, int f16, void* stream, const PackGate* gate, int e4m3) {
     PGPP_REQUIRE(x && out, "x and out must be device pointers");
     PGPP_REQUIRE(parts >= 1 && parts <= 3, "parts must be 1, 2 or 3");
     PGPP_REQUIRE(c_pad >= size[1] && c_pad % 16 == 0, "c_pad must be a multiple of 16 and >= C");
@@ -799,7 +811,7 @@ int pgpp::pack_slice(const void* x, const int64_t size[4], const int64_t stride[
     p.c_total = c_total; p.c_off = c_off;
     p.x = x; p.scale = scale; p.out = (__nv_bfloat16*)out;
     p.n = (int)size[0]; p.c = (int)size[1]; p.h = (int)size[2]; p.w = (int)size[3];
-    p.c_pad = c_pad; p.parts = parts; p.f16 = f16;
+    p.c_pad = c_pad; p.parts = parts; p.f16 = f16; p.e4m3 = e4m3;
     p.s_n = stride[0]; p.s_c = stride[1]; p.s_h = stride[2]; p.s_w = stride[3];
     p.part_stride = (long long)p.n * p.h * p.w * c_total;
     p.gate = nullptr; p.act = PGPP_ACT_LINEAR; p.alpha = 0.f; p.gain = 1.f; p.clamp = -1.f; p.csum = nullptr;

@@ -64,6 +64,29 @@ __device__ __forceinline__ void umma_bf16_lh(uint32_t tmem_d, uint32_t a_lo, uin
                  "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %5, p;\n\t}"
                  ::"r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate) : "memory");
 }
+// e4m3 operands: kind::f8f6f4 with A / B format E4M3 (0) in the instruction descriptor, K = 32 per instruction - the same 32 bytes of a
+// swizzle row as the 16 elements of kind::f16, so descriptors advance exactly as for bf16
+__device__ __forceinline__ void umma_f8(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
+    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}"
+                 ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
+}
+__device__ __forceinline__ void umma_f8_lh(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t idesc,
+                                           uint32_t accumulate) {
+    asm volatile("{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\tsetp.ne.b32 p, %6, 0;\n\tmov.b64 da, {%1, %2};\n\tmov.b64 db, {%3, %4};\n\t"
+                 "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], da, db, %5, p;\n\t}"
+                 ::"r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate) : "memory");
+}
+// F8: the operands are e4m3 bytes; otherwise bf16 / f16 (the format is in idesc)
+template <bool F8>
+__device__ __forceinline__ void umma(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
+    if constexpr (F8) umma_f8(tmem_d, desc_a, desc_b, idesc, accumulate);
+    else umma_bf16(tmem_d, desc_a, desc_b, idesc, accumulate);
+}
+template <bool F8>
+__device__ __forceinline__ void umma_lh(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t idesc, uint32_t accumulate) {
+    if constexpr (F8) umma_f8_lh(tmem_d, a_lo, a_hi, b_lo, b_hi, idesc, accumulate);
+    else umma_bf16_lh(tmem_d, a_lo, a_hi, b_lo, b_hi, idesc, accumulate);
+}
 // arrives on the mbarrier once every previously issued tcgen05.mma of this thread has completed
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");

@@ -89,7 +89,7 @@ __global__ void __launch_bounds__(256) pack_weights_kernel(WPackArgs a, long lon
             m[0] = make_float4(v[0], v[1], v[2], v[3]);
             m[1] = make_float4(v[4], v[5], v[6], v[7]);
         }
-        for (int part = 0; part < a.parts; part++) {
+        for (int part = 0; part < (a.out ? a.parts : 0); part++) {
             __align__(16) uint16_t q[8];
             #pragma unroll
             for (int j = 0; j < 8; j++) {
@@ -105,6 +105,43 @@ __global__ void __launch_bounds__(256) pack_weights_kernel(WPackArgs a, long lon
             }
             *reinterpret_cast<uint4*>(a.out + part * a.part_stride + dst) = *reinterpret_cast<const uint4*>(q);
         }
+    }
+}
+
+// e4m3 weights with one scale per GEMM column (pgpp_quantize_weights_e4m3): one CTA per (column g, sample n).  Pass 1: absmax over
+// every tap and channel of the column; pass 2: bytes = e4m3(v / scale), four channels per 32-bit store.
+__global__ void __launch_bounds__(256) quantize_weights_e4m3_kernel(const float* __restrict__ master, const float* __restrict__ s, int taps,
+                                                                    int o_rows, int c_pad, int c_in, uint8_t* __restrict__ out,
+                                                                    float* __restrict__ scale) {
+    __shared__ float s_red[8];
+    const int g = blockIdx.x, n = blockIdx.y;
+    const int q4 = c_pad >> 2, total = taps * q4;
+    auto value = [&](int t, int c) -> float {
+        if (c >= c_in) return 0.f;
+        const float m = master[((long long)t * o_rows + g) * c_pad + c];
+        return s ? m * s[(long long)n * c_in + c] : m;
+    };
+    float amax = 0.f;
+    for (int e = threadIdx.x; e < total; e += blockDim.x) {
+        const int t = e / q4, c = (e - t * q4) * 4;
+        #pragma unroll
+        for (int j = 0; j < 4; j++) amax = fmaxf(amax, fabsf(value(t, c + j)));
+    }
+    #pragma unroll
+    for (int m = 16; m > 0; m >>= 1) amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, m));
+    if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = amax;
+    __syncthreads();
+    amax = s_red[0];
+    for (int w = 1; w < 8; w++) amax = fmaxf(amax, s_red[w]);
+    const float sc = __fdiv_rn(amax, 448.f);
+    if (threadIdx.x == 0) scale[(long long)n * o_rows + g] = sc;
+    uint8_t* dst = out + (long long)n * taps * o_rows * c_pad;
+    for (int e = threadIdx.x; e < total; e += blockDim.x) {
+        const int t = e / q4, c = (e - t * q4) * 4;
+        float v[4];
+        #pragma unroll
+        for (int j = 0; j < 4; j++) v[j] = sc > 0.f ? __fdiv_rn(value(t, c + j), sc) : 0.f;
+        *reinterpret_cast<uint32_t*>(dst + ((long long)t * o_rows + g) * c_pad + c) = e4m3x4(v[0], v[1], v[2], v[3]);
     }
 }
 
@@ -151,7 +188,7 @@ extern "C" int pgpp_pack_weights(const void* w, int w_dtype, const int64_t w_siz
                                  float scale, int phases, int phase_stride, const float* fir, int flip_filter,
                                  void* out, float* master, int parts, int operand_f16, int o_rows, int o_off, int c_pad, void* stream) {
     using namespace pgpp;
-    PGPP_REQUIRE(w && out, "w and out must be device pointers");
+    PGPP_REQUIRE(w && (out || master), "w and out (or master) must be device pointers");
     PGPP_REQUIRE(w_dtype >= 0 && w_dtype <= 3, "unsupported weight dtype");
     PGPP_REQUIRE(parts >= 1 && parts <= 3 && (!operand_f16 || parts == 1), "parts must be 1..3 (1 for fp16 operands)");
     PGPP_REQUIRE(c_pad >= 8 && c_pad % 8 == 0, "c_pad must be a positive multiple of 8");
@@ -198,6 +235,21 @@ extern "C" int pgpp_up2_weight_adjoint(const float* grad_polyphase, const float*
     const long long cap = (long long)sm_count() * 8;
     if (blocks > cap) blocks = cap;
     up2_weight_adjoint_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(a);
+    count_launch();
+    PGPP_CUDA_OK(cudaGetLastError());
+    return PGPP_OK;
+}
+
+extern "C" int pgpp_quantize_weights_e4m3(const float* master, const float* s, int n, int taps, int o_rows, int c_pad, int c_in,
+                                          void* out, float* scale, void* stream) {
+    using namespace pgpp;
+    PGPP_REQUIRE(master && out && scale, "master, out and scale must be device pointers");
+    PGPP_REQUIRE(n >= 1 && n <= 65535 && taps >= 1 && o_rows >= 1 && c_pad >= 16 && c_pad % 16 == 0 && c_in >= 1 && c_in <= c_pad,
+                 "bad quantize_weights_e4m3 arguments");
+    PGPP_REQUIRE(s != nullptr || n == 1, "shared weights (s == NULL) need n == 1");
+    PGPP_REQUIRE(((uintptr_t)out & 3) == 0, "out must be 4-byte aligned");
+    quantize_weights_e4m3_kernel<<<dim3((unsigned)o_rows, (unsigned)n), 256, 0, (cudaStream_t)stream>>>(master, s, taps, o_rows, c_pad, c_in,
+                                                                                                         (uint8_t*)out, scale);
     count_launch();
     PGPP_CUDA_OK(cudaGetLastError());
     return PGPP_OK;

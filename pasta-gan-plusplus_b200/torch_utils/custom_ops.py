@@ -23,7 +23,7 @@ _LIB_PATH = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file_
 _lib = None
 _cached_plugins = dict()
 
-_DTYPES = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2, torch.float64: 3}
+_DTYPES = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2, torch.float64: 3, torch.float8_e4m3fn: 4}
 
 c_i64x4 = ctypes.c_int64 * 4
 
@@ -49,6 +49,7 @@ class ConvDesc(ctypes.Structure):
         ('spade_x', ctypes.c_void_p), ('spade_mean', ctypes.c_void_p), ('spade_rstd', ctypes.c_void_p), ('spade_pre_gain', ctypes.c_float),
         ('operand_f16', ctypes.c_int32),
         ('stats_ws', ctypes.c_void_p),
+        ('wscale', ctypes.c_void_p), ('operand_e4m3', ctypes.c_int32), ('reserved1', ctypes.c_int32),
     ]
 
 
@@ -83,6 +84,10 @@ def load_library():
     lib.pgpp_pack_activations_slice.argtypes = [vp, c_i64x4, c_i64x4, i32, vp, vp, i32, i32, i32, i32, vp]
     lib.pgpp_pack_activations_f16.restype = i32
     lib.pgpp_pack_activations_f16.argtypes = [vp, c_i64x4, c_i64x4, i32, vp, vp, i32, i32, i32, vp]
+    lib.pgpp_pack_activations_e4m3.restype = i32
+    lib.pgpp_pack_activations_e4m3.argtypes = [vp, c_i64x4, c_i64x4, i32, vp, vp, i32, i32, i32, vp]
+    lib.pgpp_quantize_weights_e4m3.restype = i32
+    lib.pgpp_quantize_weights_e4m3.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp, vp, vp]
     lib.pgpp_pack_weights.restype = i32
     lib.pgpp_pack_weights.argtypes = [vp, i32, c_i64x4, c_i64x4, i32, i32, f32, i32, i32, vp, i32, vp, vp, i32, i32, i32, i32, i32, vp]
     lib.pgpp_up2_weight_adjoint.restype = i32
@@ -136,7 +141,7 @@ def load_library():
 
 
 EXPORTED_SYMBOLS = ('pgpp_version', 'pgpp_last_error', 'pgpp_launch_count', 'pgpp_refresh_env', 'pgpp_bias_act', 'pgpp_upfirdn2d',
-                    'pgpp_modconv_demod_coefs', 'pgpp_pack_activations', 'pgpp_pack_activations_slice', 'pgpp_pack_activations_f16', 'pgpp_pack_act_gradient', 'pgpp_pack_act_gradient_tiles',
+                    'pgpp_modconv_demod_coefs', 'pgpp_pack_activations', 'pgpp_pack_activations_slice', 'pgpp_pack_activations_f16', 'pgpp_pack_activations_e4m3', 'pgpp_quantize_weights_e4m3', 'pgpp_pack_act_gradient', 'pgpp_pack_act_gradient_tiles',
                     'pgpp_pack_weights', 'pgpp_up2_weight_adjoint', 'pgpp_mul_reduce_hw', 'pgpp_sum_hw', 'pgpp_modulate_weights',
                     'pgpp_spade_modulate_pack', 'pgpp_mix_pack', 'pgpp_conv2d_direct', 'pgpp_fir_pack', 'pgpp_fir_packed', 'pgpp_fir_packed_act', 'pgpp_conv1x1_thin', 'pgpp_pack_im2col', 'pgpp_conv2d_igemm', 'pgpp_conv2d_igemm_stats_rows', 'pgpp_instnorm_finalize', 'pgpp_conv2d_wgrad', 'pgpp_u8_to_f32',
                     'pgpp_image_to_u8', 'pgpp_grid_sample_2d', 'pgpp_grid_sample_2d_backward')
@@ -292,14 +297,21 @@ class _ConvPlugin:
         return d
 
     @staticmethod
-    def pack_activations(x, scale, c_pad, parts, f16=False):
-        """-> [parts, N, H, W, c_pad] bfloat16 parts; with f16=True one part of IEEE half (dtype float16)"""
+    def pack_activations(x, scale, c_pad, parts, f16=False, e4m3=False):
+        """-> [parts, N, H, W, c_pad] bfloat16 parts; with f16=True one part of IEEE half (dtype float16); with e4m3=True one part of
+        e4m3 bytes (dtype float8_e4m3fn, round to nearest even, |v| > 448 saturates)"""
         lib = load_library()
         _torch_check(x.is_cuda and x.dim() == 4, 'x must be a rank-4 CUDA tensor')
         n, c, h, w = x.shape
         if scale is not None:
             scale = scale.detach().to(torch.float32).contiguous()
             _torch_check(tuple(scale.shape) == (n, c), 'scale must be [N, C]')
+        if e4m3:
+            out = torch.empty([1, n, h, w, c_pad], dtype=torch.float8_e4m3fn, device=x.device)
+            with torch.cuda.device(x.device):
+                _check(lib.pgpp_pack_activations_e4m3(_ptr(x), c_i64x4(*x.shape), c_i64x4(*x.stride()), dtype_code(x.dtype),
+                                                      _ptr(scale), _ptr(out), int(c_pad), int(c_pad), 0, _stream(x)))
+            return out
         if f16:
             out = torch.empty([1, n, h, w, c_pad], dtype=torch.float16, device=x.device)
             with torch.cuda.device(x.device):
@@ -335,21 +347,41 @@ class _ConvPlugin:
         (bfloat16 parts or one float16 part) and optionally master float32 [taps, o_rows, c_pad]; see pgpp_pack_weights"""
         lib = load_library()
         _torch_check(weight.is_cuda and weight.dim() == 4, 'weight must be a rank-4 CUDA tensor')
-        _torch_check(out.dim() == 4 and out.is_contiguous() and out.dtype in (torch.bfloat16, torch.float16) and out.shape[0] >= parts,
-                     'out must be a contiguous [parts, taps, o_rows, c_pad] 16-bit tensor')
-        _torch_check((out.dtype == torch.float16) == bool(f16), 'fp16 operands need a float16 destination (and only then)')
+        if out is None:     # master only (the e4m3 route quantizes it with quantize_weights_e4m3)
+            _torch_check(master is not None and master.dim() == 3, 'master [taps, o_rows, c_pad] is required when out is None')
+            o_rows, c_pad = int(master.shape[1]), int(master.shape[2])
+        else:
+            _torch_check(out.dim() == 4 and out.is_contiguous() and out.dtype in (torch.bfloat16, torch.float16) and out.shape[0] >= parts,
+                         'out must be a contiguous [parts, taps, o_rows, c_pad] 16-bit tensor')
+            _torch_check((out.dtype == torch.float16) == bool(f16), 'fp16 operands need a float16 destination (and only then)')
+            o_rows, c_pad = int(out.shape[2]), int(out.shape[3])
         w = weight.detach()
         if fir is not None:
             _torch_check(fir.is_cuda and fir.dtype == torch.float32 and tuple(fir.shape) == (4, 4), 'fir must be a float32 CUDA tensor [4, 4]')
             fir = fir.contiguous()
-        _torch_check(master is None or (master.dtype == torch.float32 and master.is_contiguous() and master.numel() == out[0].numel()),
+        _torch_check(master is None or (master.dtype == torch.float32 and master.is_contiguous() and (out is None or master.numel() == out[0].numel())),
                      'master must be a contiguous float32 tensor with taps * o_rows * c_pad elements')
         with torch.cuda.device(w.device):
             _check(lib.pgpp_pack_weights(_ptr(w), dtype_code(w.dtype), c_i64x4(*w.shape), c_i64x4(*w.stride()), int(bool(transpose_io)),
                                          int(bool(flip)), float(scale), int(phases), int(phase_stride), _ptr(fir), int(bool(flip_filter)),
-                                         _ptr(out), _ptr(master), int(parts), int(bool(f16)), int(out.shape[2]), int(o_off), int(out.shape[3]),
+                                         _ptr(out), _ptr(master), int(parts), int(bool(f16)), o_rows, int(o_off), c_pad,
                                          _stream(w)))
         return out
+
+    @staticmethod
+    def quantize_weights_e4m3(master, styles=None):
+        """master float32 [taps, o_rows, c_pad], styles [N, c_in] or None -> (e4m3 bytes float8_e4m3fn [N, 1, taps, o_rows, c_pad] (N = 1 for
+        shared weights), column scales float32 [N, o_rows]); see pgpp_quantize_weights_e4m3"""
+        lib = load_library()
+        _torch_check(master.dtype == torch.float32 and master.is_contiguous() and master.dim() == 3, 'master must be contiguous float32 [taps, o_rows, c_pad]')
+        taps, o_rows, c_pad = (int(v) for v in master.shape)
+        s = None if styles is None else styles.detach().to(torch.float32).contiguous()
+        n, c_in = (1, c_pad) if s is None else (int(s.shape[0]), int(s.shape[1]))
+        out = torch.empty([n, 1, taps, o_rows, c_pad], dtype=torch.float8_e4m3fn, device=master.device)
+        scale = torch.empty([n, o_rows], dtype=torch.float32, device=master.device)
+        with torch.cuda.device(master.device):
+            _check(lib.pgpp_quantize_weights_e4m3(_ptr(master), _ptr(s), n, taps, o_rows, c_pad, c_in, _ptr(out), _ptr(scale), _stream(master)))
+        return out, scale
 
     @staticmethod
     def sum_hw(a):
@@ -406,9 +438,16 @@ class _ConvPlugin:
         lib = load_library()
         n, c, h, w = x.shape
         parts, c_total = dst.shape[0], dst.shape[4]
-        _torch_check(tuple(dst.shape[1:4]) == (n, h, w) and dst.dtype == torch.bfloat16 and dst.is_contiguous(), 'bad packed destination')
+        _torch_check(tuple(dst.shape[1:4]) == (n, h, w) and dst.dtype in (torch.bfloat16, torch.float8_e4m3fn) and dst.is_contiguous(),
+                     'bad packed destination')
         if scale is not None:
             scale = scale.detach().to(torch.float32).contiguous()
+        if dst.dtype == torch.float8_e4m3fn:        # one part of e4m3 bytes
+            _torch_check(parts == 1, 'e4m3 operands are one part')
+            with torch.cuda.device(x.device):
+                _check(lib.pgpp_pack_activations_e4m3(_ptr(x), c_i64x4(*x.shape), c_i64x4(*x.stride()), dtype_code(x.dtype), _ptr(scale),
+                                                      _ptr(dst), int(c_pad), int(c_total), int(c_off), _stream(x)))
+            return dst
         with torch.cuda.device(x.device):
             _check(lib.pgpp_pack_activations_slice(_ptr(x), c_i64x4(*x.shape), c_i64x4(*x.stride()), dtype_code(x.dtype), _ptr(scale),
                                                    _ptr(dst), int(c_pad), int(c_total), int(c_off), int(parts), _stream(x)))

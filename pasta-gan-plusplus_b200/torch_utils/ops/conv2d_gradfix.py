@@ -15,6 +15,9 @@ Switches
                              'bf16x3' 6 products of 3-term bf16 splits (~fp32 accuracy, rel 1e-6)
                              'bf16x2' 3 products of 2-term splits (rel ~1e-5; default, within the 1e-4 bar)
                              'bf16'   1 product (rel ~3e-3; what bf16/fp16 tensors always use)
+                             'fp8'    opt-in, inference only: e4m3 operands on the kind::f8f6f4 MMA (activations at unit
+                                      scale, saturating at +-448; weights with one fp32 scale per GEMM column), ~3.7e-2
+                                      rel-L2 per layer.  A forward that autograd would record raises NotImplementedError.
 
 The weight gradient (conv2d_gradfix.py:135-142) is the split-K tcgen05 GEMM over the pixels of
 csrc/conv_wgrad.cu (`pgpp_conv2d_wgrad`); no library convolution is called anywhere on the path.
@@ -39,7 +42,8 @@ direct_few_tap_convs = os.environ.get('PGPP_NO_DIRECT_CONV') is None    # C*kh*k
 # bytes as the fp32 tensor in the bf16x2 mode) - sized for 180 GB of HBM3e.  False: re-pack in backward (round-1 behaviour).
 keep_packed_operands = True
 
-_PRODUCTS = {'bf16': (1, 1), 'bf16x2': (3, 2), 'bf16x3': (6, 3), 'f16': (1, 1)}    # name -> (MMA products, operand parts)
+_PRODUCTS = {'bf16': (1, 1), 'bf16x2': (3, 2), 'bf16x3': (6, 3), 'f16': (1, 1), 'fp8': (1, 1)}    # name -> (MMA products, operand parts)
+E4M3 = torch.float8_e4m3fn     # element type of the fp8 operand format
 _ACT_IDX = {'linear': 1, 'relu': 2, 'lrelu': 3, 'tanh': 4, 'sigmoid': 5, 'elu': 6, 'selu': 7, 'softplus': 8, 'swish': 9}
 _plugin = None
 trace = None        # set to a list to record (label, algorithmic FLOPs, start event, end event) per igemm launch (bench.py roofline)
@@ -82,6 +86,14 @@ def precision_for(dtype):
     return 'f16' if dtype == torch.float16 else 'bf16'
 
 
+def check_fp8_forward_only(*tensors):
+    """the fp8 precision is inference only: a float32 forward that autograd would record raises"""
+    if (fp32_precision == 'fp8' and torch.is_grad_enabled() and
+            any(t is not None and t.dtype in (torch.float32, torch.float64) and t.requires_grad for t in tensors)):
+        raise NotImplementedError("fp32_precision = 'fp8' is an inference-only mode (no gradients); run the forward under torch.no_grad() "
+                                  "or select 'bf16x3' / 'bf16x2' / 'bf16' for training")
+
+
 # ------------------------------------------------------------------------------------------------
 # operand packing (host logic; the packed weights are cached per parameter version)
 
@@ -101,12 +113,45 @@ def _split_bf16(t, parts):
 
 
 class PackedWeights:
-    """[parts, taps, o_rows, c_pad] bf16, K-major rows, ready for the TMA weight map."""
-    __slots__ = ('data', 'master', 'kh', 'kw', 'o', 'phases', 'phase_stride', 'o_rows', 'c_pad', 'c_in', 'parts', 'pad_y', 'pad_x', 'im2col', 'f16')
+    """[parts, taps, o_rows, c_pad] bf16, K-major rows, ready for the TMA weight map.  e4m3: ONE part of e4m3 bytes with the column
+    scales in `wscale` float32 [o_rows] (the weights of GEMM column g are data * wscale[g])."""
+    __slots__ = ('data', 'master', 'kh', 'kw', 'o', 'phases', 'phase_stride', 'o_rows', 'c_pad', 'c_in', 'parts', 'pad_y', 'pad_x', 'im2col', 'f16',
+                 'e4m3', 'wscale', 'e4m3_twin')
+
+
+def e4m3_weights(pw):
+    """the e4m3 form of bf16-packed weights (quantized from their float32 master rows, made once per PackedWeights): what an fp8 launch
+    uses when a caller packed its weights for the bf16 formats (the generator's packers)"""
+    if getattr(pw, 'e4m3', False):
+        return pw
+    twin = getattr(pw, 'e4m3_twin', None)
+    if twin is None:
+        assert pw.master is not None, 'fp16-packed weights have no float32 master rows'
+        _init()
+        data, ws = _plugin.quantize_weights_e4m3(pw.master.reshape(-1, pw.o_rows, pw.c_pad))
+        twin = PackedWeights()
+        for k in PackedWeights.__slots__:
+            if k != 'e4m3_twin':
+                setattr(twin, k, getattr(pw, k, None))
+        twin.data, twin.wscale, twin.parts, twin.e4m3, twin.f16, twin.e4m3_twin = data[0], ws[0], 1, True, False, None
+        pw.e4m3_twin = twin
+    return twin
+
+
+def e4m3_operand(x):
+    """e4m3 copy of a one-part bf16 PackedAct (the hand-over format of the generator's route, which stays bf16 across its FIR, copy, mix and
+    thin-conv kernels): the explicit bf16 -> e4m3 edge in front of an fp8 launch, one pgpp_pack_activations_e4m3 pass over the channel slice"""
+    assert x.data.dtype == torch.bfloat16 and x.data.shape[0] == 1, 'the fp8 precision converts one-part bf16 operands only'
+    _init()
+    src = x.data[0, :, :, :, x.c_off:x.c_off + x.c].permute(0, 3, 1, 2)
+    out = PackedAct(_plugin.pack_activations(src, None, _round_up(x.c, 64), 1, e4m3=True), x.c, 0, logical_hw=x.logical_hw)
+    out.im2col = x.im2col
+    return out
 
 
 class PackedAct:
-    """Activations in the tensor-core operand format: data [parts, N, H, W, c_total] bf16, channels innermost; the
+    """Activations in the tensor-core operand format: data [parts, N, H, W, c_total] bf16 (fp8 precision: one part of e4m3,
+    dtype float8_e4m3fn), channels innermost; the
     logical tensor is channels [c_off, c_off + c) of every pixel.  Convolutions can write this format directly from
     their epilogue (`out_packed=`) and read it without a packing pass."""
     __slots__ = ('data', 'c', 'c_off', 'logical_hw', 'im2col')
@@ -117,13 +162,13 @@ class PackedAct:
         self.im2col = None                  # im2col parameters when this operand was kept for the weight gradient (_forward_conv)
 
     @staticmethod
-    def empty(n, h, w, c_total, parts, device):
+    def empty(n, h, w, c_total, parts, device, dtype=torch.bfloat16):
         """buffer with c_total rounded up to whole 64-channel swizzle rows; padding channels are zeroed (they meet zero weights,
         but must not hold NaN/Inf bit patterns)"""
         c_alloc = _round_up(c_total, 64)
         if c_alloc == c_total:
-            return torch.empty([parts, n, h, w, c_alloc], dtype=torch.bfloat16, device=device)
-        return torch.zeros([parts, n, h, w, c_alloc], dtype=torch.bfloat16, device=device)
+            return torch.empty([parts, n, h, w, c_alloc], dtype=dtype, device=device)
+        return torch.zeros([parts, n, h, w, c_alloc], dtype=dtype, device=device)
 
     @property
     def shape(self):
@@ -191,6 +236,7 @@ def pack_weights(w_taps, o, phases, kh, kw, parts, pad_y, pad_x):
     pw.pad_y, pw.pad_x = pad_y, pad_x
     pw.im2col = None
     pw.f16 = False
+    pw.e4m3, pw.wscale = False, None
     return pw
 
 
@@ -205,10 +251,11 @@ def weight_layout(o, ic, phases=1):
 
 
 def pack_weights_native(weights, kh, kw, parts, pad_y, pad_x, *, transpose_io=False, flip=False, scale=1.0, up2_filter=None, flip_filter=False,
-                        f16=False):
+                        f16=False, e4m3=False):
     """PackedWeights from one weight tensor - or several stacked along the output channels (gamma | beta of a SPADE block) - in ONE
     kernel launch per tensor (pgpp_pack_weights): scale, flip, transposition, padding, bf16 split / fp16 copy, and with `up2_filter`
-    the polyphase form of the up=2 layer.  No library op touches the weights."""
+    the polyphase form of the up=2 layer.  No library op touches the weights.  e4m3: the float32 rows are quantized to e4m3 with one
+    scale per GEMM column (pgpp_quantize_weights_e4m3)."""
     _init()
     weights = list(weights) if isinstance(weights, (list, tuple)) else [weights]
     dims = [(int(w.shape[1]), int(w.shape[0])) if transpose_io else (int(w.shape[0]), int(w.shape[1])) for w in weights]
@@ -223,13 +270,18 @@ def pack_weights_native(weights, kh, kw, parts, pad_y, pad_x, *, transpose_io=Fa
     dt = torch.float16 if f16 else torch.bfloat16
     alloc = torch.zeros if o_rows != cols else torch.empty          # rows beyond the tensor must read as zero weights
     pw = PackedWeights()
-    pw.data = alloc([parts, taps, o_rows, c_pad], dtype=dt, device=dev)
+    pw.data = None if e4m3 else alloc([parts, taps, o_rows, c_pad], dtype=dt, device=dev)
     master = None if f16 else alloc([taps, o_rows, c_pad], dtype=torch.float32, device=dev)
     o_off = 0
     for w, (wo, _) in zip(weights, dims):
         _plugin.pack_weights(w, pw.data, master, transpose_io=transpose_io, flip=flip, scale=scale, phases=phases, phase_stride=phase_stride,
                              fir=up2_filter, flip_filter=flip_filter, parts=parts, f16=f16, o_off=o_off)
         o_off += wo
+    pw.e4m3, pw.wscale = bool(e4m3), None
+    if e4m3:
+        assert parts == 1 and not f16
+        data, ws = _plugin.quantize_weights_e4m3(master)
+        pw.data, pw.wscale = data[0], ws[0]
     pw.master = None if master is None else master.reshape(taps * o_rows, c_pad)
     pw.c_in = ic
     pw.kh, pw.kw, pw.o, pw.phases, pw.o_rows, pw.c_pad, pw.parts = (3, 3, o, 4, o_rows, c_pad, parts) if phases > 1 else (kh, kw, o, 1, o_rows, c_pad, parts)
@@ -279,7 +331,7 @@ def im2col_rows(ic, kh, kw):
     return r if (kh - 1) // r * r <= 6 else 0
 
 
-def packed_plain(weight, flip_weight, parts, pad_y, pad_x, transpose_io=False, scale=1.0, allow_im2col=False, f16=False):
+def packed_plain(weight, flip_weight, parts, pad_y, pad_x, transpose_io=False, scale=1.0, allow_im2col=False, f16=False, e4m3=False):
     """weight [O, I, kh, kw] used as a correlation kernel (flip_weight=True, F.conv2d semantics) or a true
     convolution kernel (flip_weight=False).  transpose_io: weight is [I, O, kh, kw] (conv_transpose2d layout).
     scale: constant folded into the packed copy (the layers' runtime weight_gain, networks.py:155,169)."""
@@ -288,8 +340,8 @@ def packed_plain(weight, flip_weight, parts, pad_y, pad_x, transpose_io=False, s
         r = im2col_rows(ic, kh, kw) if allow_im2col else 0
         if not r:
             return pack_weights_native(weight, kh, kw, parts, pad_y, pad_x, transpose_io=transpose_io, flip=not flip_weight, scale=float(scale),
-                                       f16=f16)
-        assert not f16
+                                       f16=f16, e4m3=e4m3)
+        assert not f16 and not e4m3
         w = weight.detach().to(torch.float32) * float(scale)
         if transpose_io:
             w = w.transpose(0, 1)
@@ -305,13 +357,14 @@ def packed_plain(weight, flip_weight, parts, pad_y, pad_x, transpose_io=False, s
             pw = pack_weights(wp.reshape(groups, o, r * kw * ic), o, 1, groups, 1, parts, 0, 0)
             pw.im2col = dict(r=r, kw=kw, kh=kh, pad_x=pad_x, pad_y=pad_y)
             return pw
-    return _cached(weight, ('plain', bool(flip_weight), parts, pad_y, pad_x, bool(transpose_io), float(scale), bool(allow_im2col), bool(f16)), build)
+    return _cached(weight, ('plain', bool(flip_weight), parts, pad_y, pad_x, bool(transpose_io), float(scale), bool(allow_im2col), bool(f16)) +
+                   (('e4m3',) if e4m3 else ()), build)
 
 
 _UP2_TAPS = ((2, 0), (1,))      # phase r of a stride-2 transposed 3-tap convolution: T[2j + r] = sum_t x[j + t - pad_r] * w[_UP2_TAPS[r][t]], pad_0 = 1, pad_1 = 0
 
 
-def packed_up2_phase(weight, ry, rx, flip_weight, parts):
+def packed_up2_phase(weight, ry, rx, flip_weight, parts, e4m3=False):
     """Phase (ry, rx) of `conv_transpose2d(x, w', stride=2)` for a 3 x 3 kernel as a correlation over the INPUT grid (w' = the kernel as
     conv_transpose2d sees it, conv2d_resample.py:131-132):  T[2j + ry, 2i + rx] = sum_{ty, tx} x[j + ty - (1 - ry), i + tx - (1 - rx)] * w'[KY[ty], KX[tx]]
     with KY = (2, 0) for ry = 0 and (1,) for ry = 1: 2 x 2, 2 x 1, 1 x 2 and 1 x 1 taps - the nine taps of the kernel, each used once."""
@@ -323,11 +376,11 @@ def packed_up2_phase(weight, ry, rx, flip_weight, parts):
         ky = torch.tensor(_UP2_TAPS[ry], device=w.device)
         kx = torch.tensor(_UP2_TAPS[rx], device=w.device)
         sub = w.index_select(2, ky).index_select(3, kx).contiguous()
-        return pack_weights_native(sub, len(_UP2_TAPS[ry]), len(_UP2_TAPS[rx]), parts, 1 - ry, 1 - rx)
-    return _cached(weight, ('up2_phase', ry, rx, bool(flip_weight), parts), build)
+        return pack_weights_native(sub, len(_UP2_TAPS[ry]), len(_UP2_TAPS[rx]), parts, 1 - ry, 1 - rx, e4m3=e4m3)
+    return _cached(weight, ('up2_phase', ry, rx, bool(flip_weight), parts) + (('e4m3',) if e4m3 else ()), build)
 
 
-def packed_up2_taps4(weight, flip_weight, parts):
+def packed_up2_taps4(weight, flip_weight, parts, e4m3=False):
     """`conv_transpose2d(x, w', stride=2)` for a 3 x 3 kernel as ONE 2 x 2 correlation over the input grid with 4 * O GEMM columns (phase-major,
     phase = 2 ry + rx writes T[2j + ry, 2i + rx]): tap (dy, dx) of the 2 x 2 window (padding 1) carries w'[KY, KX] for the phases that use that
     input offset and zeros for the others - 16 instead of the algorithmic 9 MACs per input pixel and (output, input) channel pair (the polyphase
@@ -345,10 +398,10 @@ def packed_up2_taps4(weight, flip_weight, parts):
                 for ty, ky in enumerate(_UP2_TAPS[ry]):
                     for tx, kx in enumerate(_UP2_TAPS[rx]):
                         w4[2 * ry + rx, :, :, ty + ry, tx + rx] = w[:, :, ky, kx]      # odd phases use only the window offset 1 (the pixel itself)
-        pw = pack_weights_native(w4.reshape(4 * o, ic, 2, 2), 2, 2, parts, 1, 1)
+        pw = pack_weights_native(w4.reshape(4 * o, ic, 2, 2), 2, 2, parts, 1, 1, e4m3=e4m3)
         pw.phases, pw.o, pw.phase_stride = 4, o, o
         return pw
-    return _cached(weight, ('up2_taps4', bool(flip_weight), parts), build)
+    return _cached(weight, ('up2_taps4', bool(flip_weight), parts) + (('e4m3',) if e4m3 else ()), build)
 
 
 def up2_modconv_packed(xp, weight, styles, dcoef, f, flip_weight, out_packed, *, noise=None, bias=None, act='linear', alpha=0.0, gain=1.0, clamp=-1.0,
@@ -360,19 +413,20 @@ def up2_modconv_packed(xp, weight, styles, dcoef, f, flip_weight, out_packed, *,
     _init()
     n, _, h, w = xp.shape
     parts = xp.data.shape[0]
+    e4m3 = xp.data.dtype == E4M3        # e4m3 GEMMs; the intermediate and the blur pass stay in bf16 (one part)
     o = weight.shape[0]
     if taps4:
         # `taps4`: the four phases as ONE 2 x 2 GEMM with 4 * O columns (16 / 9 of the algorithmic MACs, the input read once) - for the layers
         # where four passes over the input cost more than the extra MACs.  Its grid is (H + 1) x (W + 1), so the intermediate has 2H + 2 rows, the
         # last one zero (x[H] is outside the image): it stands in for the blur's bottom / right padding.
         t = PackedAct(PackedAct.empty(n, 2 * h + 2, 2 * w + 2, o, parts, xp.device), o)
-        igemm_conv(xp, packed_up2_taps4(weight, flip_weight, parts), scale=styles, dcoef=dcoef, out_hw=(h + 1, w + 1), out_packed=t)
+        igemm_conv(xp, packed_up2_taps4(weight, flip_weight, parts, e4m3), scale=styles, dcoef=dcoef, out_hw=(h + 1, w + 1), out_packed=t)
         pad = (1, 0, 1, 0)
     else:
         t = PackedAct(PackedAct.empty(n, 2 * h + 1, 2 * w + 1, o, parts, xp.device), o)
         for ry in (0, 1):
             for rx in (0, 1):
-                pw = packed_up2_phase(weight, ry, rx, flip_weight, parts)
+                pw = packed_up2_phase(weight, ry, rx, flip_weight, parts, e4m3)
                 igemm_conv(xp, pw, scale=styles, dcoef=dcoef, out_hw=(h + 1 - ry, w + 1 - rx), out_packed=t, out_phase=(ry, rx))
         pad = (1, 1, 1, 1)
     taps, fw, fh = host_filter(f)
@@ -384,7 +438,7 @@ def up2_modconv_packed(xp, weight, styles, dcoef, f, flip_weight, out_packed, *,
     return out_packed
 
 
-def packed_up2(weight, f, flip_weight, flip_filter, parts):
+def packed_up2(weight, f, flip_weight, flip_filter, parts, e4m3=False):
     """Polyphase form of `conv_transpose2d(stride=2)` followed by the 4x4 FIR with gain 4
     (conv2d_resample.py:125-139, the StyleGAN2 up=2 layer): for output pixel (2y+py, 2x+px)
 
@@ -395,8 +449,8 @@ def packed_up2(weight, f, flip_weight, flip_filter, parts):
     replaces the transposed convolution, its (2H+1)^2 intermediate and the blur pass."""
     def build():
         assert tuple(weight.shape[2:]) == (3, 3) and tuple(f.shape) == (4, 4) and f.dtype == torch.float32
-        return pack_weights_native(weight, 3, 3, parts, 1, 1, flip=bool(flip_weight), up2_filter=f, flip_filter=bool(flip_filter))
-    return _cached(weight, ('up2', bool(flip_weight), bool(flip_filter), parts), build, also=(f,))
+        return pack_weights_native(weight, 3, 3, parts, 1, 1, flip=bool(flip_weight), up2_filter=f, flip_filter=bool(flip_filter), e4m3=e4m3)
+    return _cached(weight, ('up2', bool(flip_weight), bool(flip_filter), parts) + (('e4m3',) if e4m3 else ()), build, also=(f,))
 
 
 _host_filter_cache = dict()     # id(filter tensor) -> (weakref, (data_ptr, _version), (taps, fw, fh))
@@ -465,18 +519,31 @@ def igemm_conv(x, pw, *, scale=None, stride=1, out_hw=None, dcoef=None, noise=No
     precision = precision or precision_for(src_dtype)
     products, parts = _PRODUCTS[precision]
     f16 = precision == 'f16'
+    e4m3 = precision == 'fp8'
+    esize = 1 if e4m3 else 2        # bytes per operand element
+    converted = False
+    if e4m3:        # operands packed for the bf16 formats take the explicit bf16 -> e4m3 edge
+        pw = e4m3_weights(pw)
+        if isinstance(x, PackedAct) and x.data.dtype != E4M3:
+            x, converted = e4m3_operand(x), True
     assert pw.parts >= parts, 'weights were packed with fewer parts than the requested precision needs'
     assert bool(pw.f16) == f16, 'fp16 operands need fp16-packed weights (and only they)'
+    assert bool(getattr(pw, 'e4m3', False)) == e4m3, 'e4m3 operands need e4m3-packed weights (and only they)'
     d = custom_ops.ConvDesc()
     keep = []
     if isinstance(x, PackedAct):
-        assert x.data.shape[0] >= parts and x.c_off % 8 == 0
+        assert x.data.shape[0] >= parts and x.c_off % (16 if e4m3 else 8) == 0
+        assert (x.data.dtype == E4M3) == e4m3, 'the fp8 precision takes e4m3 operands (and only it)'
         assert pw.c_pad <= x.data.shape[4] - x.c_off, 'packed activations have fewer channels than the weights expect'
-        d.act = x.data.data_ptr() + 2 * x.c_off
+        d.act = x.data.data_ptr() + esize * x.c_off
         d.a_parts = x.data.shape[0]
         d.act_pixel_stride = x.data.shape[4]
         device = x.data.device
-        if scale is not None:       # style modulation folded into per-sample weights (needs >= 128 pixels per sample)
+        if scale is not None and e4m3:      # per-sample weights: e4m3 bytes and column scales of master * styles
+            wdata, wsc = _plugin.quantize_weights_e4m3(pw.master.reshape(-1, pw.o_rows, pw.c_pad), scale)
+            keep += [wdata, wsc]
+            d.wgt = wdata.data_ptr(); d.b_parts = 1; d.wgt_per_sample = 1; d.wscale = wsc.data_ptr()
+        elif scale is not None:       # style modulation folded into per-sample weights (needs >= 128 pixels per sample)
             wdata = _plugin.modulate_weights(pw.master, scale, parts)
             keep.append(wdata)
             d.wgt = wdata.data_ptr(); d.b_parts = parts; d.wgt_per_sample = 1
@@ -486,12 +553,18 @@ def igemm_conv(x, pw, *, scale=None, stride=1, out_hw=None, dcoef=None, noise=No
         if im is not None:
             x_packed = _plugin.pack_im2col(x, scale, im['kw'], im['r'], im['pad_x'], im['pad_y'], parts)
             h = x_packed.shape[2]
+            if e4m3:        # the row-group im2col operand is packed in bf16, then takes the bf16 -> e4m3 edge
+                x_packed = e4m3_operand(PackedAct(x_packed, x_packed.shape[4])).data
         else:
-            x_packed = _plugin.pack_activations(x, scale, pw.c_pad, parts, f16=f16)
+            x_packed = _plugin.pack_activations(x, scale, pw.c_pad, parts, f16=f16, e4m3=e4m3)
         keep.append(x_packed)
         d.act = x_packed.data_ptr(); d.a_parts = parts
         d.wgt = pw.data.data_ptr(); d.b_parts = pw.data.shape[0]
         device = x.device
+    if e4m3:
+        d.operand_e4m3 = 1
+        if not d.wgt_per_sample:
+            d.wscale = pw.wscale.data_ptr()
     up = 2 if pw.phases == 4 else 1
     if out_hw is None:
         conv_h = (h + 2 * pw.pad_y - pw.kh) // stride + 1
@@ -505,8 +578,8 @@ def igemm_conv(x, pw, *, scale=None, stride=1, out_hw=None, dcoef=None, noise=No
         assert out_packed.data.shape[1] == n and 2 * (out_h - 1) + ry < th_ and 2 * (out_w - 1) + rx < tw_ and out_packed.c == pw.o
         assert pw.o % 16 == 0 and out_packed.c_off % 8 == 0 and up == 1 and spade is None
         c_total = out_packed.data.shape[4]
-        d.out = out_packed.data.data_ptr() + 2 * (out_packed.c_off + (ry * tw_ + rx) * c_total)
-        d.out_dtype = custom_ops.dtype_code(torch.bfloat16)
+        d.out = out_packed.data.data_ptr() + out_packed.data.element_size() * (out_packed.c_off + (ry * tw_ + rx) * c_total)
+        d.out_dtype = custom_ops.dtype_code(out_packed.data.dtype)
         d.out_stride = (ctypes.c_int64 * 4)(th_ * tw_ * c_total, 1, 2 * tw_ * c_total, 2 * c_total)
         d.out_parts = out_packed.data.shape[0]
         d.out_part_stride = out_packed.data[0].numel()
@@ -515,8 +588,8 @@ def igemm_conv(x, pw, *, scale=None, stride=1, out_hw=None, dcoef=None, noise=No
         assert tuple(out_packed.data.shape[1:4]) == (n, out_h, out_w) and out_packed.c == (pw.o // 2 if spade is not None else pw.o)
         assert pw.o % 16 == 0 and out_packed.c_off % 8 == 0
         c_total = out_packed.data.shape[4]
-        d.out = out_packed.data.data_ptr() + 2 * out_packed.c_off
-        d.out_dtype = custom_ops.dtype_code(torch.bfloat16)
+        d.out = out_packed.data.data_ptr() + out_packed.data.element_size() * out_packed.c_off
+        d.out_dtype = custom_ops.dtype_code(out_packed.data.dtype)      # bf16 parts, or e4m3 from e4m3 operands
         d.out_stride = (ctypes.c_int64 * 4)(out_h * out_w * c_total, 1, out_w * c_total, c_total)
         d.out_parts = out_packed.data.shape[0]
         d.out_part_stride = out_packed.data[0].numel()
@@ -596,8 +669,9 @@ def igemm_conv(x, pw, *, scale=None, stride=1, out_hw=None, dcoef=None, noise=No
         flops = 2.0 * n * pw.o * real_ic * real_taps * conv_h * conv_w
         kname = f'k{pw.kh}' if im is None else f"k{im['kh']}(im2col r{im['r']})"
         okind = ('spade' if spade is not None else 'packed' if out_packed is not None else 'nchw') + ('+acc' if accumulate else '')
-        ikind = 'packed' if isinstance(x, PackedAct) else 'tensor'
-        trace.append((f'igemm {real_ic}->{pw.o} {kname} {h}x{w}->{out_h}x{out_w} n{n} {precision} {ikind}->{okind}', flops, e0, e1))
+        ikind = ('packed(bf16->e4m3)' if converted else 'packed') if isinstance(x, PackedAct) else 'tensor'
+        elem = f'{precision}(e4m3)' if e4m3 else precision         # the operand element type that ran
+        trace.append((f'igemm {real_ic}->{pw.o} {kname} {h}x{w}->{out_h}x{out_w} n{n} {elem} {ikind}->{okind}', flops, e0, e1))
     else:
         _plugin.conv2d_igemm(d, device)
     if out_packed is None and want_f64:
@@ -631,6 +705,7 @@ def conv2d(input, weight, bias=None, stride=1, padding=0, dilation=1, groups=1, 
     comes out of the convolution's epilogue instead of a second pass over the result; its gradient is bias_act's own gradient op on the
     saved output, so first and second order gradients are those of conv2d followed by bias_act."""
     if _should_use_custom_op(input):
+        check_fp8_forward_only(input, weight, bias)
         if epilogue is not None:
             act, alpha, gain, clamp = epilogue
             assert act in FUSED_EPILOGUE_ACTS
@@ -644,6 +719,7 @@ def conv2d(input, weight, bias=None, stride=1, padding=0, dilation=1, groups=1, 
 
 def conv_transpose2d(input, weight, bias=None, stride=1, padding=0, output_padding=0, groups=1, dilation=1, weight_scale=1.0):
     if _should_use_custom_op(input):
+        check_fp8_forward_only(input, weight, bias)
         return _conv2d_gradfix(transpose=True, weight_shape=weight.shape, stride=stride, padding=padding,
                                output_padding=output_padding, groups=groups, dilation=dilation, weight_scale=float(weight_scale)).apply(input, weight, bias)
     return torch.nn.functional.conv_transpose2d(input=input, weight=_library_weight(input, weight, weight_scale), bias=bias, stride=stride,
@@ -654,7 +730,7 @@ def pack_operand(x, prec=None):
     """NCHW (or any-strided) tensor -> PackedAct in the operand format of `prec` (channels padded to whole 64-channel rows)"""
     _init()
     prec = prec or precision_for(x.dtype)
-    data = _plugin.pack_activations(x, None, _round_up(x.shape[1], 64), _PRODUCTS[prec][1], f16=prec == 'f16')
+    data = _plugin.pack_activations(x, None, _round_up(x.shape[1], 64), _PRODUCTS[prec][1], f16=prec == 'f16', e4m3=prec == 'fp8')
     return PackedAct(data, x.shape[1])
 
 
@@ -689,7 +765,7 @@ def _forward_conv(x, weight, bias, stride, padding, keep=False, scale=1.0, epi=N
     epi = epi or {}
     src_dtype = (torch.float16 if x.data.dtype == torch.float16 else weight.dtype) if isinstance(x, PackedAct) else x.dtype   # f16 operands: fp16 layer
     prec = precision_for(src_dtype)
-    im = _im2col_plan(x, weight, stride, padding) if prec != 'f16' else None
+    im = _im2col_plan(x, weight, stride, padding) if prec not in ('f16', 'fp8') else None
     if im is not None:
         # few-channel convolution: all taps of r filter rows go into the channel dimension (pgpp_pack_im2col); the operand is kept for the
         # weight gradient, which runs on it too
@@ -705,7 +781,7 @@ def _forward_conv(x, weight, bias, stride, padding, keep=False, scale=1.0, epi=N
             xp.im2col = im
             return y, xp
         return y
-    pw = packed_plain(weight, True, _PRODUCTS[prec][1], padding[0], padding[1], f16=prec == 'f16', scale=scale)
+    pw = packed_plain(weight, True, _PRODUCTS[prec][1], padding[0], padding[1], f16=prec == 'f16', scale=scale, e4m3=prec == 'fp8')
     xp, mf = x, None
     if keep and not isinstance(x, PackedAct):
         mf = torch.channels_last if (x.stride(1) == 1 and x.shape[1] > 1) else torch.contiguous_format     # the output follows the input's layout
@@ -749,7 +825,7 @@ def _conv_transpose_stride2_phases(x, weight, bias, padding, output_padding, sca
     ic, oc, kh, kw = (int(v) for v in weight.shape)
     src_dtype = (torch.float16 if x.data.dtype == torch.float16 else weight.dtype) if isinstance(x, PackedAct) else x.dtype
     prec = precision_for(src_dtype)
-    parts, f16 = _PRODUCTS[prec][1], prec == 'f16'
+    parts, f16, e4m3 = _PRODUCTS[prec][1], prec == 'f16', prec == 'fp8'
     xp = x if isinstance(x, PackedAct) else pack_operand(x, prec)
     n, _, h, w = xp.shape
     out_h = (h - 1) * 2 - 2 * padding[0] + kh + output_padding[0]
@@ -767,8 +843,10 @@ def _conv_transpose_stride2_phases(x, weight, bias, padding, output_padding, sca
             continue
         def build(ph=ph):
             sub = weight.detach()[:, :, ph['t0y']::2, ph['t0x']::2].contiguous()
-            return pack_weights_native(sub, ph['ty'], ph['tx'], parts, ph['pad_y'], ph['pad_x'], transpose_io=True, flip=True, scale=float(scale), f16=f16)
-        pw = _cached(weight, ('tconv_phase', ph['ry'], ph['rx'], int(padding[0]), int(padding[1]), parts, f16, float(scale)), build)
+            return pack_weights_native(sub, ph['ty'], ph['tx'], parts, ph['pad_y'], ph['pad_x'], transpose_io=True, flip=True, scale=float(scale), f16=f16,
+                                       e4m3=e4m3)
+        pw = _cached(weight, ('tconv_phase', ph['ry'], ph['rx'], int(padding[0]), int(padding[1]), parts, f16, float(scale)) + (('e4m3',) if e4m3 else ()),
+                     build)
         igemm_conv(xp, pw, out_hw=(int(view.shape[2]), int(view.shape[3])), out=view, bias=bias, precision=prec)
     if src_dtype == torch.float64:
         y = y.to(torch.float64)
@@ -795,7 +873,8 @@ def _forward_conv_transpose(x, weight, bias, stride, padding, output_padding, ke
     py, px = kh - 1 - padding[0], kw - 1 - padding[1]
     assert py >= 0 and px >= 0, 'conv_transpose2d padding larger than kernel_size-1 is not supported'
     prec = precision_for(src_dtype)
-    pw = packed_plain(weight, False, _PRODUCTS[prec][1], py, px, transpose_io=True, f16=prec == 'f16', scale=scale)    # flipped + transposed = equivalent correlation kernel
+    pw = packed_plain(weight, False, _PRODUCTS[prec][1], py, px, transpose_io=True, f16=prec == 'f16', scale=scale,    # flipped + transposed =
+                      e4m3=prec == 'fp8')                                                                                # equivalent correlation kernel
     n, _, h, w = x.shape
     out_h = h + 2 * py - kh + 1 + output_padding[0]
     out_w = w + 2 * px - kw + 1 + output_padding[1]

@@ -119,10 +119,11 @@ def _conv2d_resample(x, w, f, up, down, padding, groups, flip_weight, flip_filte
     # fused polyphase form of the up=2 layer (inference): one implicit-GEMM launch
     if (up == 2 and down == 1 and groups == 1 and (kh, kw) == (3, 3) and f is not None and f.ndim == 2 and (fw, fh) == (4, 4)
             and pad.fir == [1, 1, 1, 1] and conv2d_gradfix._should_use_custom_op(x) and not _needs_grad(x, w) and x.dtype != torch.float16):
-        _, parts = conv2d_gradfix._PRODUCTS[conv2d_gradfix.precision_for(x.dtype)]
+        prec = conv2d_gradfix.precision_for(x.dtype)
+        _, parts = conv2d_gradfix._PRODUCTS[prec]
         if w_scale != 1.0:
             w = w * w_scale
-        return conv2d_gradfix.igemm_conv(x, conv2d_gradfix.packed_up2(w, f, flip_weight, flip_filter, parts))
+        return conv2d_gradfix.igemm_conv(x, conv2d_gradfix.packed_up2(w, f, flip_weight, flip_filter, parts, e4m3=prec == 'fp8'))
 
     pad.widen(fw, fh, up, down)
     fir = lambda t, **kw_: upfirdn2d.upfirdn2d(x=t, f=f, flip_filter=flip_filter, **kw_)

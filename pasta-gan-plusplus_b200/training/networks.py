@@ -66,7 +66,10 @@ def modulated_conv2d_fused_act(x, weight, styles, noise=None, up=1, padding=0, r
     gain = float(spec.def_gain if gain is None else gain)
     clamp = float(-1 if clamp is None else clamp)
     src_dtype = torch.float32 if isinstance(x, conv2d_gradfix.PackedAct) else x.dtype
-    _, parts = conv2d_gradfix._PRODUCTS[conv2d_gradfix.precision_for(src_dtype)]
+    prec = conv2d_gradfix.precision_for(src_dtype)
+    _, parts = conv2d_gradfix._PRODUCTS[prec]
+    e4m3 = prec == 'fp8'        # e4m3 operands; the per-phase up = 2 form keeps its intermediate in bf16
+    conv2d_gradfix.check_fp8_forward_only(x if isinstance(x, torch.Tensor) else None, weight, styles, bias)
     dcoef = None
     if demodulate:
         conv2d_gradfix._init()
@@ -87,14 +90,14 @@ def modulated_conv2d_fused_act(x, weight, styles, noise=None, up=1, padding=0, r
             if not isinstance(x, conv2d_gradfix.PackedAct):
                 conv2d_gradfix._init()
                 ic = x.shape[1]
-                xp = conv2d_gradfix.PackedAct(conv2d_gradfix._plugin.pack_activations(x, styles, -(-ic // 64) * 64, parts), ic)
+                xp = conv2d_gradfix.PackedAct(conv2d_gradfix._plugin.pack_activations(x, styles, -(-ic // 64) * 64, parts, e4m3=e4m3), ic)
                 st = None
             return conv2d_gradfix.up2_modconv_packed(xp, weight, st, dcoef, resample_filter, flip_weight, out_packed, noise=noise, bias=bias,
                                                      act=act, alpha=alpha, gain=gain, clamp=clamp,
                                                      taps4=weight.shape[0] * weight.shape[1] < UP2_PHASES_MIN_IO)
-        pw = conv2d_gradfix.packed_up2(weight, resample_filter, flip_weight, False, parts)
+        pw = conv2d_gradfix.packed_up2(weight, resample_filter, flip_weight, False, parts, e4m3=e4m3)
     else:
-        pw = conv2d_gradfix.packed_plain(weight, flip_weight, parts, padding, padding, f16=f16)
+        pw = conv2d_gradfix.packed_plain(weight, flip_weight, parts, padding, padding, f16=f16, e4m3=e4m3)
     return conv2d_gradfix.igemm_conv(x, pw, scale=styles, dcoef=dcoef, noise=noise, bias=bias, act=act, alpha=alpha,
                                      gain=gain, clamp=clamp, out=out, out_dtype=out_dtype, accumulate=accumulate,
                                      memory_format=memory_format, out_packed=out_packed)
@@ -197,6 +200,8 @@ def modulated_conv2d(
     misc.assert_shape(x, [batch_size, in_channels, None, None])
     misc.assert_shape(styles, [batch_size, in_channels])
 
+    if conv2d_gradfix._should_use_custom_op(x):
+        conv2d_gradfix.check_fp8_forward_only(x, weight, styles, noise)
     # ---- sm_100a kernel path: one implicit GEMM, modulation / demodulation / noise fused ----
     if _kernel_path_ok(x, weight, styles, noise, up, down, padding, resample_filter):
         return modulated_conv2d_fused_act(x, weight, styles, noise=noise, up=up, padding=padding,

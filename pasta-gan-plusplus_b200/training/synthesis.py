@@ -49,6 +49,7 @@ def _can_fuse(x, *params):
 
 
 def _parts():
+    # 'fp8': the hand-over format stays one bf16 part; every implicit GEMM converts its operand to e4m3 (conv2d_gradfix.e4m3_operand)
     return conv2d_gradfix._PRODUCTS[conv2d_gradfix.fp32_precision][1]
 
 
