@@ -245,7 +245,7 @@ typedef struct {
      *     stats_ws float32 [3][M][o],  M = tiles * 4 warp partials, sample n owns rows [n * M / N, (n + 1) * M / N)
      * (no atomics: deterministic).  pgpp_instnorm_finalize turns them into mean / rstd.  Needs float32 NCHW output, one sample per
      * tile, conv_w and conv_h multiples of the pixel tile (16 x 8, or 8 x 16 in single-slab mode), o % 16 == 0, phases == 1, no
-     * accumulate; pgpp_conv2d_igemm_stats_rows reports M (0 = this launch cannot produce statistics). */
+     * accumulate; pgpp_conv2d_igemm_plan reports M as stats_rows (0 = this launch cannot produce statistics). */
     float* stats_ws;
     /* fp8 inference precision (operand_e4m3 != 0): act and wgt hold ONE part of e4m3 bytes (products == 1), act at unit scale, the
      * weights of GEMM column g divided by wscale[g] (wgt_per_sample: wscale[n * o_rows + g]); the epilogue multiplies the accumulator
@@ -258,9 +258,29 @@ typedef struct {
 /* Implicit-GEMM convolution on the 5th-gen tensor cores (tcgen05.mma, TMEM accumulators, TMA operand
  * loads), persistent over the SMs, with the epilogue above fused. */
 PGPP_API int pgpp_conv2d_igemm(const pgpp_conv_desc* desc, void* stream);
-/* rows M of the statistics workspace pgpp_conv2d_igemm would fill for this descriptor (stats_ws itself is ignored), 0 if the launch
- * cannot produce statistics, negative on an invalid descriptor */
-PGPP_API int64_t pgpp_conv2d_igemm_stats_rows(const pgpp_conv_desc* desc);
+
+/* The launch pgpp_conv2d_igemm would make for a descriptor, filled by the same validation and planning code and returned before
+ * any driver call (no device needed; without one the SM count is taken as 148, the B200's). */
+typedef struct {
+    int32_t reuse;                  /* 0: one activation box per tap; 1: one slab per filter column (ky reuse); 2: one slab per channel block */
+    int32_t slab9;                  /* single-slab mode on the straight-line 3 x 3 issuer (PGPP_IGEMM_SLAB9) */
+    int32_t stack;                  /* split-precision products a0 x [b0; b1] issued as one N = 2 * block_n MMA */
+    int32_t b_resident;             /* every weight tile of the column tile stays in shared memory */
+    int32_t inner, n_groups;        /* taps per K group, K groups per channel block */
+    int32_t parts;                  /* bf16 parts of each operand (1, 2, 3) */
+    int32_t kb;                     /* channels per K block */
+    int32_t tw, th, tn;             /* pixel tile: columns x rows x samples = 128 */
+    int32_t block_n;
+    int32_t a_stages, b_stages;     /* activation ring depth, weight slots (resident: the weight tile count) */
+    int64_t total_tiles;
+    int64_t grid;                   /* persistent CTAs: min(total_tiles, SM count) */
+    int32_t e4m3;                   /* e4m3 operands (kind::f8f6f4) */
+    int32_t epilogue;               /* 1: the lean operand-format epilogue; 0: the general one */
+    int32_t fast;                   /* general epilogue on its fast path (one sample per tile, gain folded into scale / shift) */
+    int32_t reserved0;
+    int64_t stats_rows;             /* rows M of the instance-norm workspace (see stats_ws), 0 if the launch cannot produce statistics */
+} pgpp_igemm_plan;
+PGPP_API int pgpp_conv2d_igemm_plan(const pgpp_conv_desc* desc, pgpp_igemm_plan* plan);
 /* mean[n, c] and rstd[n, c] = rsqrt(var + eps) (biased variance, torch.nn.InstanceNorm2d / torch.var_mean(unbiased=False)) from the
  * warp partials of pgpp_conv2d_igemm: ws float32 [3][rows][c], rows / n partials of 32 pixels per sample, merged in float64. */
 PGPP_API int pgpp_instnorm_finalize(const float* ws, int64_t rows, int n, int c, float eps, float* mean, float* rstd, void* stream);

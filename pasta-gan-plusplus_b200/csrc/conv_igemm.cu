@@ -1197,14 +1197,21 @@ igemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
 
 } // namespace pgpp
 
-namespace pgpp { static int igemm_launch(const pgpp_conv_desc* d, void* stream, long long* stats_rows_query); }
+namespace pgpp {
+static int igemm_plan(const pgpp_conv_desc* d, IgemmParams& p, pgpp_igemm_plan& plan, size_t& smem_bytes);
+static int igemm_launch(const pgpp_conv_desc* d, void* stream);
+}
 
-extern "C" int pgpp_conv2d_igemm(const pgpp_conv_desc* d, void* stream) { return pgpp::igemm_launch(d, stream, nullptr); }
+extern "C" int pgpp_conv2d_igemm(const pgpp_conv_desc* d, void* stream) { return pgpp::igemm_launch(d, stream); }
 
-extern "C" int64_t pgpp_conv2d_igemm_stats_rows(const pgpp_conv_desc* d) {
-    long long rows = 0;
-    const int rc = pgpp::igemm_launch(d, nullptr, &rows);
-    return rc == PGPP_OK ? (int64_t)rows : (int64_t)rc;
+extern "C" int pgpp_conv2d_igemm_plan(const pgpp_conv_desc* d, pgpp_igemm_plan* out) {
+    PGPP_REQUIRE(out != nullptr, "plan is NULL");
+    pgpp::IgemmParams p;
+    pgpp_igemm_plan plan;
+    size_t smem_bytes = 0;
+    const int rc = pgpp::igemm_plan(d, p, plan, smem_bytes);
+    if (rc == PGPP_OK) *out = plan;
+    return rc;
 }
 
 // mean / rstd from the warp partials (pivot, sum of deviations, sum of squared deviations over 32 pixels each): all partials have the same
@@ -1273,7 +1280,9 @@ extern "C" int pgpp_instnorm_finalize(const float* ws, int64_t rows, int n, int 
     return PGPP_OK;
 }
 
-static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* stats_rows_query) {
+// Validation and the launch plan (tile, rings, issuer and epilogue selection); touches no driver or device state, so the choice can be
+// queried and pinned without a GPU (pgpp_conv2d_igemm_plan).
+static int pgpp::igemm_plan(const pgpp_conv_desc* d, IgemmParams& p, pgpp_igemm_plan& plan, size_t& smem_bytes) {
     using namespace pgpp;
     PGPP_REQUIRE(d != nullptr, "desc is NULL");
     PGPP_REQUIRE(d->act && d->wgt && d->out, "act, wgt and out must be device pointers");
@@ -1312,10 +1321,6 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
     const int up = d->phases == 4 ? 2 : 1;
     PGPP_REQUIRE(d->out_h == d->conv_h * up && d->out_w == d->conv_w * up, "output size does not match the conv grid");
 
-    EncodeTiledFn encode = get_encode_fn();
-    if (!encode) { set_error("cuTensorMapEncodeTiled is not available from the driver"); return PGPP_ERR_CUDA; }
-
-    IgemmParams p;
     p.n = d->n; p.h = d->h; p.w = d->w; p.conv_h = d->conv_h; p.conv_w = d->conv_w;
     p.kh = d->kh; p.kw = d->kw; p.pad_y = d->pad_y; p.pad_x = d->pad_x; p.stride = d->stride;
     if (e4m3) p.kb = (d->c_pad % 128 == 0) ? 128 : ((d->c_pad % 64 == 0) ? 64 : 32);      // channels = bytes
@@ -1342,7 +1347,7 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
     const int row_ch = e4m3 ? 128 : 64;         // channels of a 128-byte row
     const bool slab2_shape = d->stride == 1 && d->kh * d->kw > 1 && d->kh * d->kw <= 64 && dil_y == 1 && d->c_pad % row_ch == 0 && d->block_n <= 64 &&
                              d->phases * d->phase_stride <= d->block_n && d->conv_w >= 8 && d->conv_h >= 16 && need_parts <= 2 &&
-                             !env.igemm_no_slab2 && !env.igemm_no_resident;
+                             !env.igemm_no_slab2 && !env.igemm_no_resident && !env.igemm_no_reuse;
     if (slab2_shape) {
         const long long stage = ((long long)slab_pitch * slab_rows2 * 128 + 1023) & ~1023ll;
         const long long n_bt = (long long)(d->c_pad / row_ch) * d->kh * d->kw * need_parts;
@@ -1401,8 +1406,12 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
     };
     const long long smem_max = 227 * 1024;
     const long long n_btiles = (long long)p.n_groups * p.num_cb * p.inner * p.parts;
+    // the unrolled 7-tap issuers and the 3-part 3-tap issuer only wait on the weight ring (igemm_kernel's ladder has no resident form of
+    // them): resident weights, loaded once, would leave them waiting for a second ring phase that never comes
+    const bool ks4 = p.kb * esize == 128;
+    const bool res_issuer = p.reuse == 2 || !(ks4 && ((p.inner == 7 && p.parts <= 2) || (p.inner == 3 && p.parts == 3)));
     p.b_resident = 0;
-    if (p.tiles_col == 1 && n_btiles <= 64 && !env.igemm_no_resident && smem_need(2, n_btiles) <= smem_max &&
+    if (res_issuer && p.tiles_col == 1 && n_btiles <= 64 && !env.igemm_no_resident && smem_need(2, n_btiles) <= smem_max &&
         p.total_tiles > sm_count()) {
         p.b_resident = 1;
         p.b_stages = (int)n_btiles;
@@ -1416,7 +1425,7 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
         while (p.b_stages < 8 && smem_need(p.a_stages, p.b_stages + 1) <= smem_max) p.b_stages++;
         while (p.a_stages < 4 && smem_need(p.a_stages + 1, p.b_stages) <= smem_max) p.a_stages++;
     }
-    const size_t smem_bytes = (size_t)smem_need(p.a_stages, p.b_stages);
+    smem_bytes = (size_t)smem_need(p.a_stages, p.b_stages);
     p.dcoef = d->dcoef; p.noise = d->noise; p.noise_stride_n = d->noise_stride_n; p.bias = d->bias;
     p.act_fn = d->act_fn; p.alpha = d->alpha; p.gain = d->gain; p.clamp = d->clamp;
     p.out = d->out; p.out_dtype = d->out_dtype; p.out_h = d->out_h; p.out_w = d->out_w;
@@ -1461,10 +1470,49 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
     const bool stats_ok = p.tn == 1 && p.fold_gain && d->out_dtype == PGPP_F32 && d->phases == 1 && !d->accumulate && !d->spade_x && d->o % 16 == 0 &&
                           d->conv_w % p.tw == 0 && d->conv_h % p.th == 0 && out_parts == 1;
     const long long stats_rows = stats_ok ? (long long)p.tiles_x * p.tiles_y * p.tiles_n * 4 : 0;
-    if (stats_rows_query) { *stats_rows_query = stats_rows; return PGPP_OK; }
-    PGPP_REQUIRE(!d->stats_ws || stats_ok, "stats_ws: this launch cannot produce instance-norm statistics (see pgpp_conv2d_igemm_stats_rows)");
+    PGPP_REQUIRE(!d->stats_ws || stats_ok, "stats_ws: this launch cannot produce instance-norm statistics (see pgpp_conv2d_igemm_plan)");
     PGPP_REQUIRE(((uintptr_t)d->stats_ws & 15) == 0, "stats_ws must be 16-byte aligned");
     p.stats_ws = d->stats_ws; p.stats_plane = stats_rows * d->o;
+
+    // lean operand-format epilogue (EPI 1) when the launch needs nothing else
+    // (e4m3 operands: the lean epilogue writes e4m3 - and is the only one that does)
+    const bool epi_packed = p.tn == 1 && p.fold_gain && d->out_dtype == (e4m3 ? PGPP_E4M3 : PGPP_BF16) && p.os_c == 1 && d->phases == 1 && !d->spade_x &&
+                            d->o % 16 == 0 && d->block_n >= 32 && ((uintptr_t)d->out & (e4m3 ? 15 : 31)) == 0 && p.os_w % 16 == 0 && p.os_h % 16 == 0 &&
+                            p.os_n % 16 == 0 && p.out_part_stride % 16 == 0 && (!env.igemm_no_lean_epilogue || e4m3);
+    PGPP_REQUIRE(d->out_dtype != PGPP_E4M3 || d->spade_x || (epi_packed && out_parts == 1 && !d->stats_ws),
+                 "e4m3 output: one part, channels-innermost, 16-byte aligned pixels, o % 16 == 0, phases == 1, one sample per tile, "
+                 "linear / relu / lrelu with gain > 0, block_n >= 32");
+    PGPP_REQUIRE(epi_packed || out_parts == 1 || !d->accumulate,
+                 "accumulating into a split (operand-format) output needs the lean epilogue: one sample per tile, linear / relu / lrelu with gain > 0, "
+                 "32-byte aligned pixels, block_n >= 32, phases == 1");
+    long long grid = p.total_tiles;
+    const int sms = sm_count();
+    if (grid > sms) grid = sms;
+
+    plan.reuse = p.reuse; plan.slab9 = p.slab9; plan.stack = p.stack; plan.b_resident = p.b_resident;
+    plan.inner = p.inner; plan.n_groups = p.n_groups; plan.parts = p.parts; plan.kb = p.kb;
+    plan.tw = p.tw; plan.th = p.th; plan.tn = p.tn; plan.block_n = p.block_n; plan.a_stages = p.a_stages; plan.b_stages = p.b_stages;
+    plan.total_tiles = p.total_tiles; plan.grid = grid;
+    plan.e4m3 = e4m3 ? 1 : 0; plan.epilogue = epi_packed ? 1 : 0; plan.fast = (p.tn == 1 && p.fold_gain) ? 1 : 0; plan.reserved0 = 0;
+    plan.stats_rows = stats_rows;
+    return PGPP_OK;
+}
+
+static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream) {
+    using namespace pgpp;
+    IgemmParams p;
+    pgpp_igemm_plan plan;
+    size_t smem_bytes = 0;
+    const int rc = igemm_plan(d, p, plan, smem_bytes);
+    if (rc != PGPP_OK) return rc;
+    EncodeTiledFn encode = get_encode_fn();
+    if (!encode) { set_error("cuTensorMapEncodeTiled is not available from the driver"); return PGPP_ERR_CUDA; }
+    const bool e4m3 = plan.e4m3 != 0;
+    const int esize = e4m3 ? 1 : 2;
+    const int pix_stride = d->act_pixel_stride > 0 ? d->act_pixel_stride : d->c_pad;
+    const int dil_y = d->dil_y > 1 ? d->dil_y : 1;
+    const int slab_pitch = 8 + d->kw - 1, slab_rows2 = 16 + d->kh - 1;
+    const unsigned row_bytes = (unsigned)(p.kb * esize);
 
     // tensor maps
     CUtensorMap map_a, map_b;
@@ -1490,14 +1538,6 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
                    CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(weights) failed with CUresult %d", (int)r); return PGPP_ERR_CUDA; }
     }
-    // lean operand-format epilogue (EPI 1) when the launch needs nothing else
-    // (e4m3 operands: the lean epilogue writes e4m3 - and is the only one that does)
-    const bool epi_packed = p.tn == 1 && p.fold_gain && d->out_dtype == (e4m3 ? PGPP_E4M3 : PGPP_BF16) && p.os_c == 1 && d->phases == 1 && !d->spade_x &&
-                            d->o % 16 == 0 && d->block_n >= 32 && ((uintptr_t)d->out & (e4m3 ? 15 : 31)) == 0 && p.os_w % 16 == 0 && p.os_h % 16 == 0 &&
-                            p.os_n % 16 == 0 && p.out_part_stride % 16 == 0 && (!env.igemm_no_lean_epilogue || e4m3);
-    PGPP_REQUIRE(d->out_dtype != PGPP_E4M3 || d->spade_x || (epi_packed && out_parts == 1 && !d->stats_ws),
-                 "e4m3 output: one part, channels-innermost, 16-byte aligned pixels, o % 16 == 0, phases == 1, one sample per tile, "
-                 "linear / relu / lrelu with gain > 0, block_n >= 32");
     {
         // once per device (the attribute is per function per context)
         static std::atomic<bool> done[64];
@@ -1511,12 +1551,8 @@ static int pgpp::igemm_launch(const pgpp_conv_desc* d, void* stream, long long* 
             if (dev >= 0 && dev < 64) done[dev].store(true, std::memory_order_release);
         }
     }
-    long long grid = p.total_tiles;
-    const int sms = sm_count();
-    if (grid > sms) grid = sms;
-    PGPP_REQUIRE(epi_packed || out_parts == 1 || !d->accumulate,
-                 "accumulating into a split (operand-format) output needs the lean epilogue: one sample per tile, linear / relu / lrelu with gain > 0, "
-                 "32-byte aligned pixels, block_n >= 32, phases == 1");
+    const long long grid = plan.grid;
+    const bool epi_packed = plan.epilogue == 1;
     if (e4m3) {
         if (epi_packed) igemm_kernel<1, true><<<(unsigned)grid, kThreads, smem_bytes, (cudaStream_t)stream>>>(map_a, map_b, p);
         else igemm_kernel<0, true><<<(unsigned)grid, kThreads, smem_bytes, (cudaStream_t)stream>>>(map_a, map_b, p);

@@ -53,6 +53,19 @@ class ConvDesc(ctypes.Structure):
     ]
 
 
+class IgemmPlan(ctypes.Structure):
+    """mirror of pgpp_igemm_plan (include/pgpp.h)"""
+    _fields_ = [
+        ('reuse', ctypes.c_int32), ('slab9', ctypes.c_int32), ('stack', ctypes.c_int32), ('b_resident', ctypes.c_int32),
+        ('inner', ctypes.c_int32), ('n_groups', ctypes.c_int32), ('parts', ctypes.c_int32), ('kb', ctypes.c_int32),
+        ('tw', ctypes.c_int32), ('th', ctypes.c_int32), ('tn', ctypes.c_int32), ('block_n', ctypes.c_int32),
+        ('a_stages', ctypes.c_int32), ('b_stages', ctypes.c_int32),
+        ('total_tiles', ctypes.c_int64), ('grid', ctypes.c_int64),
+        ('e4m3', ctypes.c_int32), ('epilogue', ctypes.c_int32), ('fast', ctypes.c_int32), ('reserved0', ctypes.c_int32),
+        ('stats_rows', ctypes.c_int64),
+    ]
+
+
 def library_path():
     return _LIB_PATH
 
@@ -122,8 +135,8 @@ def load_library():
     lib.pgpp_conv2d_direct.argtypes = [vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, i32, i32, f32, i32, f32, f32, f32, vp, vp, i32, i32, i32, vp]
     lib.pgpp_conv2d_igemm.restype = i32
     lib.pgpp_conv2d_igemm.argtypes = [ctypes.POINTER(ConvDesc), vp]
-    lib.pgpp_conv2d_igemm_stats_rows.restype = i64
-    lib.pgpp_conv2d_igemm_stats_rows.argtypes = [ctypes.POINTER(ConvDesc)]
+    lib.pgpp_conv2d_igemm_plan.restype = i32
+    lib.pgpp_conv2d_igemm_plan.argtypes = [ctypes.POINTER(ConvDesc), ctypes.POINTER(IgemmPlan)]
     lib.pgpp_instnorm_finalize.restype = i32
     lib.pgpp_instnorm_finalize.argtypes = [vp, i64, i32, i32, f32, vp, vp, vp]
     lib.pgpp_conv2d_wgrad.restype = i32
@@ -143,7 +156,7 @@ def load_library():
 EXPORTED_SYMBOLS = ('pgpp_version', 'pgpp_last_error', 'pgpp_launch_count', 'pgpp_refresh_env', 'pgpp_bias_act', 'pgpp_upfirdn2d',
                     'pgpp_modconv_demod_coefs', 'pgpp_pack_activations', 'pgpp_pack_activations_slice', 'pgpp_pack_activations_f16', 'pgpp_pack_activations_e4m3', 'pgpp_quantize_weights_e4m3', 'pgpp_pack_act_gradient', 'pgpp_pack_act_gradient_tiles',
                     'pgpp_pack_weights', 'pgpp_up2_weight_adjoint', 'pgpp_mul_reduce_hw', 'pgpp_sum_hw', 'pgpp_modulate_weights',
-                    'pgpp_spade_modulate_pack', 'pgpp_mix_pack', 'pgpp_conv2d_direct', 'pgpp_fir_pack', 'pgpp_fir_packed', 'pgpp_fir_packed_act', 'pgpp_conv1x1_thin', 'pgpp_pack_im2col', 'pgpp_conv2d_igemm', 'pgpp_conv2d_igemm_stats_rows', 'pgpp_instnorm_finalize', 'pgpp_conv2d_wgrad', 'pgpp_u8_to_f32',
+                    'pgpp_spade_modulate_pack', 'pgpp_mix_pack', 'pgpp_conv2d_direct', 'pgpp_fir_pack', 'pgpp_fir_packed', 'pgpp_fir_packed_act', 'pgpp_conv1x1_thin', 'pgpp_pack_im2col', 'pgpp_conv2d_igemm', 'pgpp_conv2d_igemm_plan', 'pgpp_instnorm_finalize', 'pgpp_conv2d_wgrad', 'pgpp_u8_to_f32',
                     'pgpp_image_to_u8', 'pgpp_grid_sample_2d', 'pgpp_grid_sample_2d_backward')
 
 
@@ -641,14 +654,13 @@ class _ConvPlugin:
             _check(lib.pgpp_conv2d_igemm(ctypes.byref(desc), stream))
 
     @staticmethod
-    def conv2d_igemm_stats_rows(desc, device):
-        """rows of the instance-norm partial workspace this launch would fill (0: it cannot produce statistics)"""
+    def conv2d_igemm_plan(desc):
+        """the launch conv2d_igemm would make for `desc` as a dict of the pgpp_igemm_plan fields (issuer, rings, epilogue, grid,
+        stats_rows = rows of the instance-norm workspace, 0 if the launch cannot produce statistics); needs no GPU"""
         lib = load_library()
-        with torch.cuda.device(device):
-            rows = int(lib.pgpp_conv2d_igemm_stats_rows(ctypes.byref(desc)))
-        if rows < 0:
-            raise RuntimeError(lib.pgpp_last_error().decode())
-        return rows
+        plan = IgemmPlan()
+        _check(lib.pgpp_conv2d_igemm_plan(ctypes.byref(desc), ctypes.byref(plan)))
+        return {name: getattr(plan, name) for name, _ in IgemmPlan._fields_ if name != 'reserved0'}
 
     @staticmethod
     def instnorm_finalize(ws, n, eps):

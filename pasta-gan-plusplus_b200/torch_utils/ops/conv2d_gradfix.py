@@ -655,7 +655,7 @@ def igemm_conv(x, pw, *, scale=None, stride=1, out_hw=None, dcoef=None, noise=No
     stats_ws = None
     if instnorm_eps is not None:
         assert out_packed is None and spade is None
-        rows = _plugin.conv2d_igemm_stats_rows(d, device) if (result.dtype == torch.float32 and result.is_contiguous()) else 0
+        rows = _plugin.conv2d_igemm_plan(d)['stats_rows'] if (result.dtype == torch.float32 and result.is_contiguous()) else 0
         if rows > 0:
             stats_ws = torch.empty([3, rows, pw.o], dtype=torch.float32, device=device)
             d.stats_ws = stats_ws.data_ptr()
