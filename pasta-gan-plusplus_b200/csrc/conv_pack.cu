@@ -137,12 +137,10 @@ __device__ __forceinline__ float act_gradient_from_output(float dy, float y, con
 
 template <class T> struct RawVec4 { typedef uint2 type; };          // 4 consecutive pixels of a 16-bit tensor
 template <> struct RawVec4<float> { typedef float4 type; };
-template <> struct RawVec4<double> { typedef float4 type; };        // never loaded (VEC is false for 64-bit sources)
 template <class T> __device__ __forceinline__ float raw_get(const typename RawVec4<T>::type& q, int k) {
     return (float)to_acc<T>(reinterpret_cast<const T*>(&q)[k]);
 }
 template <> __device__ __forceinline__ float raw_get<float>(const float4& q, int k) { return reinterpret_cast<const float*>(&q)[k]; }
-template <> __device__ __forceinline__ float raw_get<double>(const float4& q, int k) { return reinterpret_cast<const float*>(&q)[k]; }
 
 template <class T, bool VEC, bool GATE = false>
 __global__ void __launch_bounds__(256) pack_nchw_kernel(PackArgs p, TileGeom g) {
@@ -282,14 +280,19 @@ static int launch_pack(const PackArgs& p, cudaStream_t stream) {
         const long long blocks = (long long)g.x_tiles * g.y_tiles * g.c_tiles * p.n;
         PGPP_REQUIRE(blocks <= 2147483647LL, "activation tensor too large to pack");
         const size_t smem = (size_t)p.parts * 128 * 8 * sizeof(uint4);
-        // 128-bit loads: rows 16-byte aligned and either W % 4 == 0 or a row pitch that covers the last (partial) group of 4
-        const bool vec = sizeof(T) <= 4 && (p.w % 4 == 0 || p.s_h >= (p.w + 3) / 4 * 4) && p.s_c % 4 == 0 && p.s_h % 4 == 0 && p.s_n % 4 == 0 &&
-                         ((uintptr_t)p.x & (4 * sizeof(T) - 1)) == 0;
-        if (p.gate) {
-            if (vec) pack_nchw_kernel<T, true, true><<<(unsigned)blocks, 256, smem, stream>>>(p, g);
-            else pack_nchw_kernel<T, false, true><<<(unsigned)blocks, 256, smem, stream>>>(p, g);
-        } else if (vec) pack_nchw_kernel<T, true><<<(unsigned)blocks, 256, smem, stream>>>(p, g);
-        else pack_nchw_kernel<T, false><<<(unsigned)blocks, 256, smem, stream>>>(p, g);
+        if constexpr (sizeof(T) <= 4) {
+            // 128-bit loads: rows 16-byte aligned and either W % 4 == 0 or a row pitch that covers the last (partial) group of 4
+            const bool vec = (p.w % 4 == 0 || p.s_h >= (p.w + 3) / 4 * 4) && p.s_c % 4 == 0 && p.s_h % 4 == 0 && p.s_n % 4 == 0 &&
+                             ((uintptr_t)p.x & (4 * sizeof(T) - 1)) == 0;
+            if (p.gate) {
+                if (vec) pack_nchw_kernel<T, true, true><<<(unsigned)blocks, 256, smem, stream>>>(p, g);
+                else pack_nchw_kernel<T, false, true><<<(unsigned)blocks, 256, smem, stream>>>(p, g);
+            } else if (vec) pack_nchw_kernel<T, true><<<(unsigned)blocks, 256, smem, stream>>>(p, g);
+            else pack_nchw_kernel<T, false><<<(unsigned)blocks, 256, smem, stream>>>(p, g);
+        } else {
+            // 64-bit sources: element loads only, and no gate (pgpp_pack_act_gradient takes 16- and 32-bit dtypes)
+            pack_nchw_kernel<T, false><<<(unsigned)blocks, 256, smem, stream>>>(p, g);
+        }
     } else {
         PGPP_REQUIRE(!p.gate, "pgpp_pack_act_gradient needs pixel-contiguous (NCHW) tensors");
         const long long total = (long long)p.n * p.h * p.w * p.c_pad;
